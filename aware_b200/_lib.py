@@ -67,6 +67,9 @@ SIGNATURES = {
     "aw_stoi_batch": (_i, [_vp, _vp, _i64, _vp, _i64, _i, _i, _vp, _vp, C.c_double, _vp]),
     "aw_stft_band": (_i, [_vp, _vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp]),
     "aw_istft_band": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
+    "aw_stft_full": (_i, [_vp, _vp, _i, _i, _i64, _vp, _vp]),
+    "aw_phase_vocoder": (_i, [_vp, _vp, _i, _i, C.c_double, _i, _vp, _vp]),
+    "aw_istft_full": (_i, [_vp, _vp, _i, _i, _i, _vp, _i64, _vp]),
     "aw_gemm": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "aw_attack_pcm": (_i, [_vp, _vp, _i, _i, _i64, _i, _vp, _i64, _vp]),
     "aw_attack_decimate_interp": (_i, [_vp, _vp, _i, _i, _i64, _i, _vp, _i64, _vp]),

@@ -6,12 +6,16 @@ Each class also has `.apply_batch(x, sr, rng)` taking a CUDA float32 tensor
 from the numpy Generator passed in (or given directly), never from global state
 (the reference draws from unseeded global RNGs, attacks.py:170,340,378).
 Filter design (scipy.signal.butter / firwin / lfilter_zi) stays on the host; only
-coefficients travel.  MP3Compression / TimeStretch / PitchShift shell out to
-ffmpeg / rubberband upstream and have no arithmetic to restate: not provided.
+coefficients travel.  Upstream's MP3Compression / TimeStretch / PitchShift shell out to
+ffmpeg / rubberband and have no arithmetic to restate.  MP3 is not provided (`CompressionApprox`
+is an in-repo stand-in); `TimeStretch` / `PitchShift` are defined here as the classical phase
+vocoder (parity unpinned to rubberband), with `desync_attacks()` as the set the evaluation
+driver adds on request.
 """
 from __future__ import annotations
 
 import math
+from fractions import Fraction
 
 import numpy as np
 import torch
@@ -361,6 +365,116 @@ class CompressionApprox(Attack):
         mag, ph = eng.stft_band(x, sr, normalize=False, phasor=True)
         delta = eng.istft_band(eng.spectral_quantize(mag, self.step_db, self.floor_db), ph, sr)
         return eng.attack_affine(x[:, :L], 1.0, delta, 1.0)
+
+
+# ---- desynchronisation attacks (upstream: rubberband, scripts/attacks.py:150-252; parity unpinned)
+RATE_MIN, RATE_MAX = 0.25, 4.0
+
+
+def check_rate(rate) -> float:
+    """The phase vocoder's rate as a float; ValueError unless it is finite and in [0.25, 4]."""
+    r = float(rate)
+    if not (math.isfinite(r) and RATE_MIN <= r <= RATE_MAX):
+        raise ValueError(f"time-stretch rate must be finite and in [{RATE_MIN:g}, {RATE_MAX:g}] (got {rate!r})")
+    return r
+
+
+def stretch_frames(n_frames: int, rate: float) -> int:
+    """Output frames of the phase vocoder: len(np.arange(0, n_frames, rate)) = ceil(n_frames / rate)."""
+    return math.ceil(n_frames / rate)
+
+
+def stretch_length(n_samples: int, rate: float) -> int:
+    """Output samples of a time stretch: round(N / rate) (librosa.effects.time_stretch)."""
+    return int(round(n_samples / rate))
+
+
+def pitch_ratio(n_steps, max_cents: float = 0.05) -> Fraction:
+    """The resampling ratio of `PitchShift`: the fraction p / q with the smallest q (p = round(q r)) within
+    `max_cents` of r = 2^(n_steps / 12).  At 0.05 cents, +-2 semitones give 55/49 and 49/55, and no q
+    exceeds 433 for |n_steps| <= 12.  (Fraction(r).limit_denominator(256) misses 0.05 cents at +-5 and
+    +-7 semitones, by up to 1.4 cents.)"""
+    r = 2.0 ** (float(n_steps) / 12.0)
+    if not (math.isfinite(r) and max_cents > 0):
+        raise ValueError("pitch_ratio: n_steps must be finite and max_cents > 0")
+    q = 1
+    while True:
+        p = max(1, round(r * q))
+        if abs(1200.0 * math.log2(p / (q * r))) <= max_cents:
+            return Fraction(p, q)
+        q += 1
+
+
+def _time_stretch(eng, x, rate):
+    spec = eng.stft_full(x)
+    return eng.istft_full(eng.phase_vocoder(spec, rate), stretch_length(x.shape[1], rate))
+
+
+class TimeStretch(Attack):
+    """Time stretch by `rate` without changing pitch -- PARITY UNPINNED: upstream calls rubberband, whose
+    engine (transient detection, phase locking) has no arithmetic to follow, so the attack is defined here
+    as the classical phase vocoder of librosa.effects.time_stretch in this project's STFT conventions:
+
+      D     = torch.stft(x, 1024, 256, window=hann_window(1024), center=True)   (reflect pad, all 513
+              bins, the float32 input as it is, no peak normalisation), T = 1 + N // 256 frames
+      out   = librosa.phase_vocoder(D, rate, hop_length=256) with every operation in float64
+              (DESIGN.md section 7 spells it out), rounded to complex64, ceil(T / rate) frames
+      y     = torch.istft(out, 1024, 256, window, center=True, length=round(N / rate))
+
+    rate > 1 gives shorter, faster audio (pyrubberband's convention); rate must lie in [0.25, 4].
+    Stages: Engine.stft_full / phase_vocoder / istft_full.  Pinned by its numpy restatement
+    (tests/desync_oracle.py) in tests/test_desync_attacks.py."""
+
+    def __init__(self, rate):
+        self.rate = check_rate(rate)
+        self.name = f"time_stretch_{rate}"
+
+    def apply_batch(self, x, sr, rng=None, engine=None):
+        eng = _eng(engine)
+        return _time_stretch(eng, eng._audio(x), self.rate)
+
+
+class PitchShift(Attack):
+    """Pitch shift by `n_steps` semitones at constant length -- PARITY UNPINNED (upstream: rubberband), defined
+    as librosa.effects.pitch_shift's construction on the phase vocoder of `TimeStretch`:
+
+      1. time-stretch by rate 2^(-n_steps / 12) (n_steps > 0: longer audio);
+      2. resample by q / p, where p / q = pitch_ratio(n_steps, max_cents) approximates 2^(n_steps / 12):
+         scipy.signal.resample_poly(y, q, p), the bit-exact polyphase kernel of `Resample` (skipped when p = q);
+      3. truncate or zero-pad to the input length N.
+
+    n_steps > 0 raises the pitch; |n_steps| <= 24 (the stretch rate stays in [0.25, 4])."""
+
+    def __init__(self, n_steps, max_cents=0.05):
+        self.n_steps = n_steps
+        self.rate = check_rate(2.0 ** (-float(n_steps) / 12.0))
+        self.ratio = pitch_ratio(n_steps, max_cents)
+        self.name = f"pitch_shift_{n_steps}"
+        self._plans = {}
+
+    def apply_batch(self, x, sr, rng=None, engine=None):
+        eng = _eng(engine)
+        x = eng._audio(x)
+        n = x.shape[1]
+        y = _time_stretch(eng, x, self.rate)
+        p, q = self.ratio.numerator, self.ratio.denominator
+        if p != q:
+            key = (y.shape[1], eng.device.index)
+            if key not in self._plans:
+                h_tf, tpp, first, n_res = polyphase_plan(y.shape[1], q, p)
+                self._plans[key] = (torch.from_numpy(h_tf).to(eng.device), tpp, first, n_res)
+            h, tpp, first, n_res = self._plans[key]
+            y = eng.attack_upfirdn(y, h, tpp, q, p, first, n_res)
+        if y.shape[1] >= n:
+            return y[:, :n]
+        return torch.nn.functional.pad(y, (0, n - y.shape[1]))
+
+
+def desync_attacks():
+    """The desynchronisation attacks `evaluate_clips(..., desync=True)` appends.  Upstream's time-stretch
+    and pitch-shift parameters are not recorded in this repository; these values are this project's
+    choice: +-10 % tempo and +-2 semitones."""
+    return [TimeStretch(0.9), TimeStretch(1.1), PitchShift(-2), PitchShift(2)]
 
 
 def reference_suite():

@@ -23,6 +23,7 @@
 #include "spec.cuh"
 #include "spectc.cuh"
 #include "stoi.cuh"
+#include "vocoder.cuh"
 
 namespace aw {
 thread_local char g_err[512] = "";
@@ -2309,6 +2310,81 @@ extern "C" int aw_istft_band(aw_ctx* ctx, const float* d_mag, const float* d_pha
   s.amp = d_mag; s.ph = (const float2*)d_phasor; s.scale = 1.0f / AW_NFFT;
   s.y_oob = (float*)ctx->yoob.p; s.y = d_wave; s.peak_y = acc.peak_y;
   return launch_syn<SYN_WAVE>(ctx, d, s, st);
+}
+
+// full-band STFT / phase vocoder / iSTFT (time-stretch and pitch-shift attacks): no band, no peak, no
+// synchronisation and nothing staged on the host
+extern "C" int aw_stft_full(aw_ctx* ctx, const float* d_audio, int n_clips, int n_samples, int64_t stride,
+                            float* d_spec, void* stream) {
+  AW_REQUIRE(ctx && d_audio && d_spec, "null argument");
+  AW_REQUIRE(n_clips >= 1 && n_clips <= 65535, "aw_stft_full: n_clips must be in [1, 65535] (got %d)", n_clips);
+  AW_REQUIRE(n_samples > AW_NFFT, "aw_stft_full: clips must be longer than 1024 samples (got %d)", n_samples);
+  AW_REQUIRE(stride >= n_samples, "aw_stft_full: stride must be >= n_samples");
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  AnaArgs a;
+  memset(&a, 0, sizeof(a));
+  a.sig = d_audio; a.sig_stride = stride; a.len = n_samples;
+  a.T = 1 + n_samples / AW_HOP; a.bin0 = 0; a.nbins = AW_NBINS_FULL;
+  a.window = ctx->d_window; a.twiddle = ctx->d_twiddle; a.env256 = ctx->d_env256;
+  a.ph = (float2*)d_spec;
+  if (raise_smem_limit(ctx, (const void*)k_analysis<ANA_FULL, 0, 16>, AW_ANA_SMEM)) return 1;
+  dim3 g((a.T + AW_ANA_FRAMES - 1) / AW_ANA_FRAMES, n_clips);
+  prof_mark(ctx, st, "stft_full");
+  k_analysis<ANA_FULL, 0, 16><<<g, 128, AW_ANA_SMEM, st>>>(a);
+  ctx->launches++;
+  AW_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int aw_phase_vocoder(aw_ctx* ctx, const float* d_spec, int n_clips, int n_frames, double rate,
+                                int n_frames_out, float* d_out, void* stream) {
+  AW_REQUIRE(ctx && d_spec && d_out, "null argument");
+  AW_REQUIRE(std::isfinite(rate) && rate >= 0.25 && rate <= 4.0,
+             "aw_phase_vocoder: rate must be finite and in [0.25, 4] (got %g)", rate);
+  AW_REQUIRE(n_clips >= 1 && n_frames >= 1, "aw_phase_vocoder: n_clips and n_frames must be >= 1");
+  const double want = ceil((double)n_frames / rate);        // len(np.arange(0, n_frames, rate))
+  AW_REQUIRE((double)n_frames_out == want, "aw_phase_vocoder: n_frames_out must be ceil(n_frames / rate) = %.0f (got %d)",
+             want, n_frames_out);
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long threads = (long long)n_clips * AW_NBINS_FULL;
+  prof_mark(ctx, st, "phase_vocoder");
+  k_phase_vocoder<<<(unsigned)((threads + 127) / 128), 128, 0, st>>>((const float2*)d_spec, n_clips, n_frames, rate,
+                                                                      n_frames_out, (float2*)d_out);
+  ctx->launches++;
+  AW_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int aw_istft_full(aw_ctx* ctx, const float* d_spec, int n_clips, int n_frames, int n_out,
+                             float* d_wave, int64_t out_stride, void* stream) {
+  AW_REQUIRE(ctx && d_spec && d_wave, "null argument");
+  AW_REQUIRE(n_clips >= 1 && n_clips <= 65535, "aw_istft_full: n_clips must be in [1, 65535] (got %d)", n_clips);
+  AW_REQUIRE(n_frames >= 1, "aw_istft_full: n_frames must be >= 1 (got %d)", n_frames);
+  AW_REQUIRE(n_out >= 1, "aw_istft_full: n_out must be >= 1 (got %d)", n_out);
+  AW_REQUIRE(out_stride >= n_out, "aw_istft_full: out_stride must be >= n_out");
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  // samples past 256 (n_frames - 1) + 512 lie outside every frame: torch.istft pads them with zeros
+  const int n_ola = std::min(n_out, AW_HOP * (n_frames - 1) + AW_HALF);
+  SynArgs s;
+  memset(&s, 0, sizeof(s));
+  s.ph = (const float2*)d_spec; s.T = n_frames; s.L = n_out; s.bin0 = 0; s.nbins = AW_NBINS_FULL;
+  s.scale = 1.0f / AW_NFFT;
+  s.window = ctx->d_window; s.twiddle = ctx->d_twiddle; s.env256 = ctx->d_env256;
+  s.y = d_wave; s.x_stride = out_stride;
+  // (the bin-group template arguments select the band loader, which this mode does not use)
+  if (raise_smem_limit(ctx, (const void*)k_synthesis<SYN_FULL, 0, 15>, AW_SYN_SMEM)) return 1;
+  const int hops = (AW_HALF + n_ola + AW_HOP - 1) / AW_HOP;   // padded-axis hops holding the output samples
+  dim3 g((hops + AW_SYN_HOPS - 1) / AW_SYN_HOPS, n_clips);
+  prof_mark(ctx, st, "istft_full");
+  k_synthesis<SYN_FULL, 0, 15><<<g, 128, AW_SYN_SMEM, st>>>(s);
+  ctx->launches++;
+  AW_LAUNCH_CHECK();
+  if (n_out > n_ola)
+    AW_CUDA(cudaMemset2DAsync(d_wave + n_ola, (size_t)out_stride * 4, 0, (size_t)(n_out - n_ola) * 4, n_clips, st));
+  return 0;
 }
 
 extern "C" int aw_gemm(aw_ctx* ctx, const float* d_a, const float* d_b, float* d_d, int rows, int n,

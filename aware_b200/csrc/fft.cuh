@@ -138,6 +138,10 @@ struct NadamStep {
 // analysis: frames -> band spectrum
 // ---------------------------------------------------------------------------
 enum { ANA_MAG = 0, ANA_INIT = 1, ANA_CPLX = 2 };   // CPLX: complex band spectrum only (spectc.cuh's S_oob)
+// FULL: all 513 bins of the input as it is (no peak scaling), complex, for aw_stft_full; bin0 = 0,
+// nbins = AW_NBINS_FULL, instantiated over k2 = 0..16 (lane 0 of k2 = 16 is the Nyquist bin, its own mirror)
+enum { ANA_FULL = 3 };
+#define AW_NBINS_FULL 513
 
 struct AnaArgs {
   const float* sig;            // per clip signal x
@@ -182,11 +186,15 @@ __global__ void __launch_bounds__(128, 3) k_analysis(AnaArgs a) {
   // ---- stage the (scaled / padded) signal segment -------------------------
   const float* sig = a.sig + (long long)clip * a.sig_stride;
   const int m_end = AW_HOP * (T - 1) + AW_NFFT;   // padded length
-  const unsigned long long pk = a.peak[clip];
-  const float p1 = peak_value(pk);
-  const float d1 = p1 + 1e-8f;
-  const float d2 = __fdiv_rn(p1, d1) + 1e-8f;
-  {
+  if (MODE == ANA_FULL) {
+    for (int j = tid; j < AW_ANA_SIG; j += 128) {
+      const int m = AW_HOP * t0 + j;
+      s_sig[j] = m < m_end ? sig[reflect_idx(m - AW_HALF, L)] : 0.f;
+    }
+  } else {
+    const unsigned long long pk = a.peak[clip];
+    const float p1 = peak_value(pk);
+    const float d1 = p1 + 1e-8f;
     // x / d1 as one multiply by the correctly rounded reciprocal (<= 1 ulp from the division)
     const float inv = __fdiv_rn(1.0f, d1);
     for (int j = tid; j < AW_ANA_SIG; j += 128) {
@@ -221,7 +229,8 @@ __global__ void __launch_bounds__(128, 3) k_analysis(AnaArgs a) {
       // brev5(31-k2) of lane 32-lane (lane > 0) or register brev5(32-k2) of lane 0.
       float mr = __shfl_sync(0xffffffffu, re[brev5(31 - k2)], src);
       float mi = __shfl_sync(0xffffffffu, im[brev5(31 - k2)], src);
-      if (k2 >= 1 && lane == 0) {
+      // (lane 0 of k2 = 0 is the DC bin, its own mirror: only the full spectrum contains it)
+      if ((k2 >= 1 || MODE == ANA_FULL) && lane == 0) {
         mr = re[brev5((32 - k2) & 31)];
         mi = im[brev5((32 - k2) & 31)];
       }
@@ -236,7 +245,7 @@ __global__ void __launch_bounds__(128, 3) k_analysis(AnaArgs a) {
         if (f == 1 && !has_b) break;
         const long long o = ((long long)clip * T + (ta + f)) * a.nbins + b;
         const float sr = fr[f], si = fi[f];
-        if (MODE == ANA_CPLX) {
+        if (MODE == ANA_CPLX || MODE == ANA_FULL) {
           a.ph[o] = make_float2(sr, si);
         } else {
           const float mag = sqrtf(sr * sr + si * si);
@@ -261,6 +270,9 @@ __global__ void __launch_bounds__(128, 3) k_analysis(AnaArgs a) {
 // synthesis: band spectrum -> windowed overlap-add
 // ---------------------------------------------------------------------------
 enum { SYN_OOB = 0, SYN_WAVE = 1 };   // the loop passes live in spec.cuh
+// FULL: torch.istft(spec, length=L) of a full complex spectrum (`ph`: [clip][T][AW_NBINS_FULL], no `amp`,
+// no y_oob, no peak) into y with row stride x_stride (aw_istft_full)
+enum { SYN_FULL = 2 };
 
 struct SynArgs {
   const float* amp;            // [clip][T][nbins] real factor (c / cbest / dA~)
@@ -270,7 +282,7 @@ struct SynArgs {
   const float* window;
   const float2* twiddle;       // layout [k1][lane]
   const float* env256;
-  // SYN_OOB: y_oob = x/(peak_x+1e-8) - ola/env
+  // SYN_OOB: y_oob = x/(peak_x+1e-8) - ola/env  (SYN_FULL: x_stride is the row stride of y, x is unused)
   const float* x; long long x_stride; const unsigned long long* peak_x;
   float* y_oob;                // [clip][L]   (OOB: out; WAVE: in)
   float* z_oob;                // [clip][L]   (OOB: optional out) y_oob * envelope, for spec.cuh
@@ -338,6 +350,60 @@ __device__ __forceinline__ void syn_pair(const SynArgs& a, int clip, int ta, int
   }
 }
 
+// syn_pair for a full spectrum: all 513 bins, complex.  As irfft does, the imaginary parts of the DC and
+// Nyquist bins are ignored.  Lane l holds Z[l + 32 k2] (k2 = 0..15) in register k2 and the mirrored
+// entries Z[1024 - k'] in registers 16..31; lane 0's register 16 is the Nyquist bin Z[512].
+__device__ __forceinline__ void syn_pair_full(const SynArgs& a, int clip, int ta, int tb, bool va, bool vb,
+                                              float (&re)[32], float (&im)[32], float2* my_tr,
+                                              const float2* s_tw, const float* s_win, int lane) {
+  const float2* xa = a.ph + ((long long)clip * a.T + (va ? ta : 0)) * AW_NBINS_FULL;
+  const float2* xb = a.ph + ((long long)clip * a.T + (vb ? tb : 0)) * AW_NBINS_FULL;
+  const float sa = va ? a.scale : 0.f, sb = vb ? a.scale : 0.f;
+  const int lm = (32 - lane) & 31;
+#pragma unroll
+  for (int k2 = 0; k2 < 16; ++k2) {
+    {
+      float2 p0 = xa[lane + 32 * k2], p1 = xb[lane + 32 * k2];
+      if (k2 == 0 && lane == 0) { p0.y = 0.f; p1.y = 0.f; }
+      const float ar = sa * p0.x, ai = sa * p0.y, br = sb * p1.x, bi = sb * p1.y;
+      re[k2] = ar - bi;
+      im[k2] = ai + br;
+    }
+    {
+      const float2 p0 = xa[lm + 32 * k2], p1 = xb[lm + 32 * k2];
+      const float ar = sa * p0.x, ai = sa * p0.y, br = sb * p1.x, bi = sb * p1.y;
+      const float zr = ar + bi, zi = br - ai;
+      if (lane == 0) {
+        if (k2 >= 1) { re[32 - k2] = zr; im[32 - k2] = zi; }
+      } else {
+        re[31 - k2] = zr;
+        im[31 - k2] = zi;
+      }
+    }
+  }
+  if (lane == 0) {
+    re[16] = sa * xa[512].x;
+    im[16] = sb * xb[512].x;
+  }
+  warp_fft1024<1>(re, im, my_tr, s_tw, lane);
+#pragma unroll
+  for (int p = 0; p < 32; ++p) {
+    const float w = s_win[lane + 32 * brev5(p)];
+    re[p] *= w;
+    im[p] *= w;
+  }
+}
+
+template <int MODE, int K2LO, int K2HI>
+__device__ __forceinline__ void syn_frames(const SynArgs& a, int clip, int ta, int tb, bool va, bool vb,
+                                           float (&re)[32], float (&im)[32], float2* my_tr,
+                                           const float2* s_tw, const float* s_win, int lane) {
+  if (MODE == SYN_FULL)
+    syn_pair_full(a, clip, ta, tb, va, vb, re, im, my_tr, s_tw, s_win, lane);
+  else
+    syn_pair<K2LO, K2HI>(a, clip, ta, tb, va, vb, re, im, my_tr, s_tw, s_win, lane);
+}
+
 __device__ __forceinline__ void ola_add(float* s_ola, int off, const float (&v)[32], int lane) {
 #pragma unroll
   for (int p = 0; p < 32; ++p) s_ola[off + lane + 32 * brev5(p)] += v[p];
@@ -383,7 +449,7 @@ __global__ void __launch_bounds__(128, 2) k_synthesis(SynArgs a) {
     const int ta = fw + 2 * pr, tb = ta + 1;
     const bool va = ta >= 0 && ta < T, vb = tb >= 0 && tb < T;
     if (!(va || vb)) continue;                     // warp-uniform
-    syn_pair<K2LO, K2HI>(a, clip, ta, tb, va, vb, re, im, my_tr, s_tw, s_win, lane);
+    syn_frames<MODE, K2LO, K2HI>(a, clip, ta, tb, va, vb, re, im, my_tr, s_tw, s_win, lane);
     if (va) ola_add(s_ola, ow + AW_HOP * (2 * pr), re, lane);
     if (pr < 2) {
       if (vb) ola_add(s_ola, ow + AW_HOP * (2 * pr + 1), im, lane);
@@ -399,7 +465,7 @@ __global__ void __launch_bounds__(128, 2) k_synthesis(SynArgs a) {
     const int ta = fw + 6, tb = ta + 1;
     const bool va = ta >= 0 && ta < T, vb = tb >= 0 && tb < T;
     if (va || vb) {
-      syn_pair<K2LO, K2HI>(a, clip, ta, tb, va, vb, re, im, my_tr, s_tw, s_win, lane);
+      syn_frames<MODE, K2LO, K2HI>(a, clip, ta, tb, va, vb, re, im, my_tr, s_tw, s_win, lane);
       if (va) ola_add(s_ola, ow + AW_HOP * 6, re, lane);
       if (vb) ola_add(s_ola, ow + AW_HOP * 7, im, lane);
     }
@@ -411,6 +477,19 @@ __global__ void __launch_bounds__(128, 2) k_synthesis(SynArgs a) {
   const int m_total = AW_HOP * (T - 1) + AW_NFFT;
   int m_hi = m_lo + AW_HOP * AW_SYN_HOPS;
   if (m_hi > m_total) m_hi = m_total;
+
+  if (MODE == SYN_FULL) {
+    // output sample n = m - 512 < L; m < m_total bounds it by 256 (T - 1) + 512, past which torch.istft
+    // pads with zeros (the caller's job).  The last 512 samples are the tail of the final frame over its
+    // small window envelope, as torch computes them.
+    float* yc = a.y + (long long)clip * a.x_stride;
+    for (int m = m_lo + tid; m < m_hi; m += 128) {
+      const int n = m - AW_HALF;
+      if (n < 0 || n >= L) continue;
+      yc[n] = s_ola[m - AW_HOP * f0] * ola_inv_envelope(m, T, s_win, a.env256);
+    }
+    return;
+  }
 
   {
     float best = -1.f;

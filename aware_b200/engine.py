@@ -7,6 +7,7 @@ aware_b200.service / .embedding / .detection is a thin layer over it.
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import numpy as np
 import torch
@@ -15,6 +16,7 @@ from . import _lib
 
 N_BITS = 20
 HOP = 256
+N_BINS_FULL = 513
 
 
 def _ptr(t):
@@ -286,6 +288,46 @@ class Engine:
         wave = torch.empty((n, HOP * (T - 1)), dtype=torch.float32, device=mag.device)
         _lib.check(self.lib.aw_istft_band(self._ctx, _ptr(mag.contiguous()), _ptr(phasor.contiguous()), n, T,
                                           int(sample_rate), _ptr(wave), _stream()))
+        return wave
+
+    @staticmethod
+    def _spectrum(spec):
+        if not (isinstance(spec, torch.Tensor) and spec.is_cuda and spec.dtype == torch.complex64 and spec.dim() == 3
+                and spec.shape[2] == N_BINS_FULL):
+            raise ValueError("expected a CUDA complex64 spectrum [n_clips, n_frames, 513]")
+        return torch.view_as_real(spec.contiguous())
+
+    def stft_full(self, audio):
+        """[n, N] -> complex64 [n, T, 513], T = 1 + N // 256: torch.stft(x, 1024, 256, hann_window(1024),
+        center=True) of every clip, all bins, the input as it is (no peak normalisation).  Frame-major: clip
+        i's torch.stft result is out[i].T."""
+        x = self._audio(audio)
+        n, N = x.shape
+        spec = torch.empty((n, 1 + N // HOP, N_BINS_FULL, 2), dtype=torch.float32, device=x.device)
+        _lib.check(self.lib.aw_stft_full(self._ctx, _ptr(x), n, N, x.stride(0), _ptr(spec), _stream()))
+        return torch.view_as_complex(spec)
+
+    def phase_vocoder(self, spec, rate):
+        """complex64 [n, T, 513] -> [n, ceil(T / rate), 513]: librosa.phase_vocoder(D, rate, hop_length=256)
+        in float64 (aw_phase_vocoder); rate finite and in [0.25, 4]."""
+        s = self._spectrum(spec)
+        n, T = s.shape[:2]
+        rate = float(rate)
+        T_out = math.ceil(T / rate) if math.isfinite(rate) and rate > 0 else 0
+        out = torch.empty((n, max(T_out, 1), N_BINS_FULL, 2), dtype=torch.float32, device=s.device)
+        _lib.check(self.lib.aw_phase_vocoder(self._ctx, _ptr(s), n, T, rate, T_out, _ptr(out), _stream()))
+        return torch.view_as_complex(out)
+
+    def istft_full(self, spec, n_out):
+        """complex64 [n, T, 513] -> float32 [n, n_out]: torch.istft(D, 1024, 256, hann_window(1024),
+        center=True, length=n_out) of every clip (imaginary parts of bins 0 and 512 ignored)."""
+        s = self._spectrum(spec)
+        n, T = s.shape[:2]
+        if int(n_out) < 1:
+            raise ValueError("n_out must be >= 1")
+        wave = torch.empty((n, int(n_out)), dtype=torch.float32, device=s.device)
+        _lib.check(self.lib.aw_istft_full(self._ctx, _ptr(s), n, T, int(n_out), _ptr(wave), wave.stride(0),
+                                          _stream()))
         return wave
 
     def gemm(self, a, b, precision=None):

@@ -9,11 +9,13 @@ Upstream does this one clip at a time on the CPU.  Here clips are grouped by len
 resample-to-16 kHz step (`scipy.signal.resample_poly(audio, 16000, sr)`, test.py:60-65) runs
 on the GPU through the same bit-exact polyphase kernel the `Resample` attack uses, and with
 `torch.distributed` initialised the per-attack error counters are all-reduced once at the end
-(`parallel.allreduce_counters`).  The MP3 / time-stretch / pitch-shift attacks need external
-binaries and PESQ / STOI third-party packages: they are used when available on the host and
-skipped otherwise, exactly like the optional `webrtcvad` gate.
+(`parallel.allreduce_counters`).  Upstream's MP3 attack calls ffmpeg and is not run.  Its
+time-stretch and pitch-shift attacks call rubberband; `desync=True` (`--desync`) appends this
+project's phase-vocoder definitions of them (`attacks.desync_attacks()`: time stretch 0.9 / 1.1,
+pitch shift -2 / +2 semitones).  STOI runs on the GPU; PESQ is a third-party package, scored
+when installed and skipped otherwise, like the optional `webrtcvad` gate.
 
-    python -m aware_b200.evaluate <folder with .wav files> [--iters 400] [--seed 0]
+    python -m aware_b200.evaluate <folder with .wav files> [--iters 400] [--seed 0] [--desync]
 """
 from __future__ import annotations
 
@@ -97,8 +99,9 @@ def bucket_by_length(lengths):
 
 
 def default_attacks(rng: np.random.Generator):
-    """The in-scope subset of test.py:15-18's list (MP3 / TimeStretch / PitchShift need external
-    binaries).  Random parameters are drawn per batch from `rng` (upstream draws them unseeded)."""
+    """The in-scope subset of test.py:15-18's list (MP3 / TimeStretch / PitchShift call external
+    binaries upstream; the latter two are available as `attacks.desync_attacks()`).  Random parameters
+    are drawn per batch from `rng` (upstream draws them unseeded)."""
     return [A.PCMBitDepthConversion(8), A.PCMBitDepthConversion(12), A.PCMBitDepthConversion(16),
             A.PCMBitDepthConversion(24), A.DeleteSamples(0.1), A.DeleteSamples(0.15), A.DeleteSamples(0.2),
             A.Resample(), A.RandomBandstop(), A.SampleSupression(0.1), A.SampleSupression(0.25),
@@ -106,16 +109,20 @@ def default_attacks(rng: np.random.Generator):
 
 
 # ------------------------------------------------------------------------------ the driver
-def evaluate_clips(clips, rates, embedder, detector, attack_list=None, seed: int = 0, keep_audio: bool = False):
+def evaluate_clips(clips, rates, embedder, detector, attack_list=None, seed: int = 0, keep_audio: bool = False,
+                   desync: bool = False):
     """clips: list of 1-D float arrays, rates: their sample rates.  Returns a dict with per-attack
     mean BER in percent ('orig' = no attack, as upstream's `rec`), mean SNR, the decoded bits and
     (optionally) the watermarked audio, all for THIS rank's shard when torch.distributed is
-    initialised -- the means are over all ranks (counter all-reduce)."""
+    initialised -- the means are over all ranks (counter all-reduce).  `desync` appends
+    `attacks.desync_attacks()` (time stretch / pitch shift) to the attack list."""
     from .service import detect_watermark_batch, embed_watermark_batch
     eng = embedder.engine
     A.set_engine(eng)
     rng = np.random.default_rng(seed)
     attack_list = default_attacks(rng) if attack_list is None else attack_list
+    if desync:
+        attack_list = list(attack_list) + A.desync_attacks()
     names = ["orig"] + [a.name for a in attack_list]
     world = torch.distributed.get_world_size() if torch.distributed.is_initialized() else 1
     rank = torch.distributed.get_rank() if torch.distributed.is_initialized() else 0
@@ -195,6 +202,8 @@ def main(argv=None):
     ap.add_argument("folder")
     ap.add_argument("--iters", type=int, default=400)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--desync", action="store_true",
+                    help="also run the time-stretch (0.9, 1.1) and pitch-shift (-2, +2 semitones) attacks")
     args = ap.parse_args(argv)
     from .utils.models import load
     paths = sorted(os.path.join(args.folder, f) for f in os.listdir(args.folder) if f.lower().endswith(".wav"))
@@ -205,7 +214,7 @@ def main(argv=None):
     embedder, detector = load()
     embedder.num_iterations = args.iters
     embedder.verbose = False
-    res = evaluate_clips(list(clips), list(rates), embedder, detector, seed=args.seed)
+    res = evaluate_clips(list(clips), list(rates), embedder, detector, seed=args.seed, desync=args.desync)
     for name, v in res["ber_percent"].items():
         logger.info(f"{name}: mean: {v:.4f}")
     logger.info(f"snr: mean: {res['snr_db_mean']:.2f} dB over {res['n_clips']} clips")

@@ -187,6 +187,27 @@ int aw_stft_band(aw_ctx* ctx, const float* d_audio, int n_clips, int n_samples, 
                  int sample_rate, int normalize, float* d_mag, float* d_phasor, void* stream);
 int aw_istft_band(aw_ctx* ctx, const float* d_mag, const float* d_phasor, int n_clips,
                   int n_frames, int sample_rate, float* d_wave, void* stream);
+
+/* ---- full-band STFT / phase vocoder / iSTFT: the stages of the time-stretch and pitch-shift attacks
+ * (parity unpinned to upstream's rubberband calls; the classical phase vocoder of
+ * librosa.effects.time_stretch, defined in DESIGN.md section 7).  Spectra are complex64, frame-major:
+ * float2 [n_clips][n_frames][513].  None of the three synchronises the stream.
+ *
+ * aw_stft_full: torch.stft(x, 1024, 256, window, center=True, pad_mode="reflect") of every clip, all 513
+ * bins, the input as it is (no peak normalisation).  n_samples > 1024; n_frames = 1 + n_samples / 256. */
+int aw_stft_full(aw_ctx* ctx, const float* d_audio, int n_clips, int n_samples, int64_t stride,
+                 float* d_spec, void* stream);
+/* aw_phase_vocoder: librosa.phase_vocoder(D, rate, hop_length=256) in float64, out rounded to complex64.
+ * rate finite and in [0.25, 4]; n_frames_out must equal ceil(n_frames / rate) (= len(np.arange(0, n_frames,
+ * rate))).  One thread per (clip, bin): results do not depend on the batch. */
+int aw_phase_vocoder(aw_ctx* ctx, const float* d_spec, int n_clips, int n_frames, double rate,
+                     int n_frames_out, float* d_out, void* stream);
+/* aw_istft_full: torch.istft(D, 1024, 256, window, center=True, length=n_out) per clip into rows of
+ * out_stride floats.  The imaginary parts of bins 0 and 512 are ignored (as irfft does); samples
+ * [256 (n_frames-1), 256 (n_frames-1) + 512) are the tail of the last frame over its window envelope,
+ * samples past that are 0.  n_out >= 1. */
+int aw_istft_full(aw_ctx* ctx, const float* d_spec, int n_clips, int n_frames, int n_out, float* d_wave,
+                  int64_t out_stride, void* stream);
 /* D[rows][N] = A[rows][K] * B[N][K]^T ; rows % 128 == 0, K % 32 == 0, N in {64,128,256,512,1024} */
 int aw_gemm(aw_ctx* ctx, const float* d_a, const float* d_b, float* d_d, int rows, int n, int k,
             int prec, void* stream);
