@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libaware_b200.so")
 
 PREC_TF32, PREC_FP32, PREC_BF16, PREC_FP16 = 0, 1, 2, 3
-OPT_THRESHOLD, OPT_EXACT_MARGIN, OPT_TC_SPECTRAL, OPT_TWO_PASS, OPT_PAIR_GEMM, OPT_BWD64_STREAM, OPT_FUSE_NORM = 0, 1, 2, 3, 4, 5, 6
+OPT_THRESHOLD, OPT_EXACT_MARGIN, OPT_TC_SPECTRAL, OPT_TWO_PASS, OPT_PAIR_GEMM, OPT_BWD64_STREAM = 0, 1, 2, 3, 4, 5
 STAT_DETECT_CLIPS, STAT_REEVAL_CLIPS = 0, 1
 SCALE_NONE, SCALE_SIGNED_MAX = 0, 1
 

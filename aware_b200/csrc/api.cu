@@ -83,8 +83,6 @@ struct aw_ctx {
   // CUDA-graph replay of the optimisation iteration (AW_B200_NO_GRAPH=1 disables): the ~50 launches
   // of one iteration are captured once on a context-owned stream and replayed iters-1 times
   bool graphs = true;
-  bool pdl = false;                // set while the optimisation loop launches (aw_launch): programmatic dependent launch
-  bool pdl_ok = false;             // AW_B200_PDL=1: on (opt-in: measured neutral to negative)
   cudaStream_t gstream = nullptr;
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;
   Buf accum, peakx, mag, ph_u, ph_q, c0, c, m, v, cbest, dA, yoob, y, M, cs, sigma;
@@ -97,14 +95,6 @@ struct aw_ctx {
   size_t h_lowm_cap = 0;
   double exact_margin = 1e-3;      // AW_OPT_EXACT_MARGIN
   bool two_pass = true;            // small-K layers as statistics pass + apply pass (AW_B200_ONE_PASS=1: off)
-  // 16-bit loops, K >= 512 layers: InstanceNorm (+ LeakyReLU) / its adjoint inside the GEMM (EPI_*_FUSE); bit 0
-  // forward, bit 1 backward (AW_OPT_FUSE_NORM, AW_B200_FUSE_NORM=<mask>); fuse_pair: on CTA pairs where pair_ok
-  // DEFAULT OFF: measured a wash to a loss at 256 clips (DESIGN.md, "InstanceNorm inside the GEMM")
-  int fuse_norm = 0;
-  bool fuse_pair = false;
-  Buf fuse_cnt;
-  int fuse_cnt_tpc = 0;
-  bool fuse_cnt_fresh = true;
   bool bwd64_stream = true;        // 16-bit loops: the backward K = 64 layer on k_gemm_bwd64 (TMA-streamed activations, AW_OPT_BWD64_STREAM)
   // tensor-core spectral path of the fp16 embed loop (spectc.cuh; AW_B200_FFT_SPEC=1: off)
   bool tc_spec = true;
@@ -175,9 +165,8 @@ static const char* gemm_label(int epi, int n, int k) {
   static char table[32][32];
   static int used = 0;
   char buf[32];
-  static const char* kind[11] = {"plain", "fwd", "bwd", "fwd_stats", "fwd_apply", "bwd_stats", "bwd_apply", "peak", "spec",
-                                 "fwd_fuse", "bwd_fuse"};
-  snprintf(buf, sizeof(buf), "gemm_%s_n%d_k%d", epi >= 0 && epi < 11 ? kind[epi] : "other", n, k);
+  static const char* kind[9] = {"plain", "fwd", "bwd", "fwd_stats", "fwd_apply", "bwd_stats", "bwd_apply", "peak", "spec"};
+  snprintf(buf, sizeof(buf), "gemm_%s_n%d_k%d", epi >= 0 && epi < 9 ? kind[epi] : "other", n, k);
   for (int i = 0; i < used; ++i)
     if (strcmp(table[i], buf) == 0) return table[i];
   if (used == 32) return "gemm_other";
@@ -192,25 +181,6 @@ static int raise_smem_limit(aw_ctx* ctx, const void* func, int bytes) {
   AW_CUDA(cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   ctx->smem_attr_done.push_back(func);
   return 0;
-}
-
-// Kernel launch on `st`.  Inside the optimisation loop (ctx->pdl) with programmatic stream serialisation: the
-// kernel may be scheduled while its predecessor drains and blocks in pdl_wait() until that one has completed
-// (every kernel launched through here starts with pdl_enter() / pdl_wait()); captured into the iteration's
-// CUDA graph as programmatic dependency edges.  Otherwise an ordinary launch.
-template <typename... KA, typename... A>
-static void aw_launch(aw_ctx* ctx, void (*kern)(KA...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                      A&&... args) {
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute at;
-  memset(&at, 0, sizeof(at));
-  at.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at.val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = &at;
-  cfg.numAttrs = ctx->pdl ? 1 : 0;
-  cudaLaunchKernelEx(&cfg, kern, KA(args)...);
 }
 
 static int ensure(Buf& b, size_t bytes) {
@@ -351,8 +321,8 @@ static int launch_tc(aw_ctx* ctx, const CUtensorMap& ma, const CUtensorMap& mb, 
     cudaEventRecord(pr.a, st);
   }
   prof_mark(ctx, st, gemm_label(EPI, n, k));
-  aw_launch(ctx, k_gemm_tc<T, OT, BN, EPI>, dim3(grid), dim3(gemm_threads(EPI)), gemm_tc_smem<BN>(), st, ma, mb, k, n_row_tiles,
-                                                                              n_col_tiles, ep);
+  k_gemm_tc<T, OT, BN, EPI><<<grid, gemm_threads(EPI), gemm_tc_smem<BN>(), st>>>(ma, mb, k, n_row_tiles,
+                                                                                 n_col_tiles, ep);
   if (ctx->prof_on) {
     cudaEventRecord(pr.b, st);
     ctx->prof.push_back(pr);
@@ -378,8 +348,8 @@ static int launch_tc_pair(aw_ctx* ctx, const CUtensorMap& ma, const CUtensorMap&
     cudaEventRecord(pr.a, st);
   }
   prof_mark(ctx, st, gemm_label(EPI, n, k));
-  aw_launch(ctx, k_gemm_tc_pair<T, OT, BN, EPI>, dim3(grid), dim3(gemm_threads(EPI)), gemm_tc_smem_pair<BN>(), st, ma, mb_half, k, n_row_tiles,
-                                                                                        n_col_tiles, ep);
+  k_gemm_tc_pair<T, OT, BN, EPI><<<grid, gemm_threads(EPI), gemm_tc_smem_pair<BN>(), st>>>(ma, mb_half, k, n_row_tiles,
+                                                                                           n_col_tiles, ep);
   if (ctx->prof_on) {
     cudaEventRecord(pr.b, st);
     ctx->prof.push_back(pr);
@@ -388,60 +358,6 @@ static int launch_tc_pair(aw_ctx* ctx, const CUtensorMap& ma, const CUtensorMap&
   AW_LAUNCH_CHECK();
   return 0;
 }
-static bool pair_ok(aw_ctx* ctx, int rows, int n, int k, int elem_bytes);
-// EPI_FWD_FUSE / EPI_BWD_FUSE (gemm.cuh): InstanceNorm (+ LeakyReLU) / its adjoint inside the GEMM.  The grid is a
-// multiple of the group size (all row tiles of a clip -- of two clips for CTA pairs with an odd tile count -- for
-// one column panel), at most one CTA per SM: the CTAs of a group are co-resident and at the same tile when they
-// exchange their column sums.  `ep` must carry tiles_per_clip, Tp, part, stat / stat_out.
-template <typename T, typename OT, int EPI, int CG>
-static int launch_tc_fused(aw_ctx* ctx, const CUtensorMap& ma, const CUtensorMap& mb, int rows, int n, int k,
-                           EpiArgsT<OT> ep, int n_clips, cudaStream_t st) {
-  constexpr int BN = 256;
-  auto kern = CG == 2 ? k_gemm_tc_pair<T, OT, BN, EPI> : k_gemm_tc<T, OT, BN, EPI>;
-  const int smem = CG == 2 ? gemm_tc_smem_pair<BN, EPI>() : gemm_tc_smem<BN>();
-  if (raise_smem_limit(ctx, (const void*)kern, smem)) return 1;
-  const int n_row_tiles = rows / 128, n_col_tiles = n / BN, tpc = ep.tiles_per_clip;
-  const int gs = CG == 2 && tpc % 2 == 0 ? tpc / 2 : tpc;       // group size in tiles (CG = 2: pair-tiles)
-  const int tiles = n_row_tiles / CG * n_col_tiles;
-  AW_REQUIRE(tiles % gs == 0 && gs <= ctx->num_sms / CG, "fused InstanceNorm GEMM: bad tile grouping (%d tiles, groups of %d)", tiles, gs);
-  const int units = std::min(tiles, ctx->num_sms / CG / gs * gs);
-  {
-    const void* before = ctx->fuse_cnt.p;
-    if (ensure(ctx->fuse_cnt, (size_t)std::max(n_clips * n_col_tiles, 1) * sizeof(unsigned))) return 1;
-    if (ctx->fuse_cnt.p != before) ctx->fuse_cnt_fresh = true;
-  }
-  if (ctx->fuse_cnt_tpc != tpc || ctx->fuse_cnt_fresh) {
-    // counters only ever advance by tiles_per_clip per launch; a new clip length (or a grown buffer) restarts them
-    AW_CUDA(cudaMemsetAsync(ctx->fuse_cnt.p, 0, ctx->fuse_cnt.cap, st));
-    ctx->fuse_cnt_tpc = tpc;
-    ctx->fuse_cnt_fresh = false;
-  }
-  ep.fuse_cnt = (unsigned*)ctx->fuse_cnt.p;
-  ep.fuse_gs = gs;
-  aw_ctx::ProfRec pr;
-  if (ctx->prof_on) {
-    pr.n = n; pr.k = k; pr.epi = EPI;
-    pr.a = prof_event(ctx); pr.b = prof_event(ctx);
-    cudaEventRecord(pr.a, st);
-  }
-  prof_mark(ctx, st, gemm_label(EPI, n, k));
-  aw_launch(ctx, kern, dim3(units * CG), dim3(gemm_threads(EPI, CG)), (size_t)smem, st, ma, mb, k, n_row_tiles, n_col_tiles, ep);
-  if (ctx->prof_on) {
-    cudaEventRecord(pr.b, st);
-    ctx->prof.push_back(pr);
-  }
-  ctx->launches++;
-  AW_LAUNCH_CHECK();
-  return 0;
-}
-// which form (0 = none, 1 = single CTAs, 2 = CTA pairs) the fused layer takes: 16-bit loops only, not in the
-// frame-sharded mode (its statistics are all-reduced over ranks between the GEMM and the apply pass)
-static int fuse_form(aw_ctx* ctx, int mask, int n_clips, int tiles_per_clip, int rows, int n, int k, int elem_bytes) {
-  if (!(ctx->fuse_norm & mask) || ctx->sh || elem_bytes != 2 || n % 256 != 0 || tiles_per_clip > 32) return 0;
-  if (ctx->fuse_pair && pair_ok(ctx, rows, n, k, elem_bytes) && (tiles_per_clip % 2 == 0 || n_clips % 2 == 0)) return 2;
-  return 1;
-}
-
 // Measured (256 clips x 10 s, profiles/r2_pair_gemm.txt): the pair wins where operand staging bounds the
 // tile -- K bytes per row >= 2 KB (TF32 K >= 512: -16 %, fp16 K = 1024: -5..10 %); at fp16 K = 512 the
 // tile is epilogue-bound and coupling the two CTAs' drains costs 15 %, so that layer stays on single CTAs.
@@ -463,8 +379,8 @@ static int launch_bwd64(aw_ctx* ctx, const CUtensorMap& ma, const CUtensorMap& m
     cudaEventRecord(pr.a, st);
   }
   prof_mark(ctx, st, gemm_label(EPI, n, k));
-  aw_launch(ctx, k_gemm_bwd64<T, EPI>, dim3(grid), dim3(320), gemm64_smem<EPI>(), st, ma, mb128, mact, mout, k,
-            n_row_tiles, n_col_tiles, ga);
+  k_gemm_bwd64<T, EPI><<<grid, 320, gemm64_smem<EPI>(), st>>>(ma, mb128, mact, mout, k,
+                                                              n_row_tiles, n_col_tiles, ga);
   if (ctx->prof_on) {
     cudaEventRecord(pr.b, st);
     ctx->prof.push_back(pr);
@@ -532,18 +448,12 @@ extern "C" int aw_ctx_create(aw_ctx** out, int device, const aw_model* model) {
   {
     const char* e = getenv("AW_B200_NO_GRAPH");
     ctx->graphs = !(e && e[0] == '1');
-    const char* e0 = getenv("AW_B200_PDL");          // measured: no gain (DESIGN.md, experiments), hence opt-in
-    ctx->pdl_ok = e0 && e0[0] == '1';
     const char* e2 = getenv("AW_B200_ONE_PASS");
     ctx->two_pass = !(e2 && e2[0] == '1');
     const char* e3 = getenv("AW_B200_FFT_SPEC");
     ctx->tc_spec = !(e3 && e3[0] == '1');
     const char* e4 = getenv("AW_B200_NO_PAIR");
     ctx->pair_gemm = !(e4 && e4[0] == '1');
-    const char* e5 = getenv("AW_B200_FUSE_NORM");
-    if (e5 && e5[0]) ctx->fuse_norm = atoi(e5) & 3;
-    const char* e6 = getenv("AW_B200_FUSE_PAIR");
-    if (e6 && e6[0]) ctx->fuse_pair = e6[0] == '1';
   }
 
   void* fn = nullptr;
@@ -692,10 +602,6 @@ extern "C" int aw_ctx_set_option(aw_ctx* ctx, int option, double value) {
     case AW_OPT_TWO_PASS: ctx->two_pass = value != 0.0; return 0;
     case AW_OPT_PAIR_GEMM: ctx->pair_gemm = value != 0.0; return 0;
     case AW_OPT_BWD64_STREAM: ctx->bwd64_stream = value != 0.0; return 0;
-    case AW_OPT_FUSE_NORM:
-      ctx->fuse_norm = (int)value & 3;
-      ctx->fuse_pair = ((int)value & 4) != 0;
-      return 0;
     default: return set_error("aw_ctx_set_option: unknown option %d", option);
   }
 }
@@ -882,7 +788,6 @@ struct Acc {
 static Acc acc_view(aw_ctx* ctx, const struct Dims& d);
 
 __global__ void k_iter_begin(unsigned long long* peak, int n, int* it, unsigned* dmax = nullptr) {
-  pdl_enter();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) peak[i] = 0ull;
   if (i < n && dmax) dmax[i] = 0u;
@@ -1072,7 +977,7 @@ static int net_forward(aw_ctx* ctx, const Dims& d, const Acc& acc, const SparseM
   {
     dim3 g((d.T + AW_MEL_FRAMES - 1) / AW_MEL_FRAMES, d.n);
     prof_mark(ctx, st, "mel");
-    aw_launch(ctx, k_mel, dim3(g), dim3(128), AW_MEL_FRAMES * d.nb * 4, st, own_frames(ctx, (float*)ctx->mag.p, d.nb), d.T, d.nb, sm,
+    k_mel<<<g, 128, AW_MEL_FRAMES * d.nb * 4, st>>>(own_frames(ctx, (float*)ctx->mag.p, d.nb), d.T, d.nb, sm,
                                                     (float*)ctx->M.p, acc.chan_part, peak_scale);
     ctx->launches++;
     AW_LAUNCH_CHECK();
@@ -1085,11 +990,11 @@ static int net_forward(aw_ctx* ctx, const Dims& d, const Acc& acc, const SparseM
       cb = 1;
     } else if (reduce_if_long(ctx, ctx->red_a, cp, cb, d.n, 2 * AW_NMEL, st)) return 1;
     prof_mark(ctx, st, "mel_stats");
-    aw_launch(ctx, k_mel_stats, dim3(d.n), dim3(128), 0, st, cp, cb, ctx->sh ? ctx->sh->T_glob : d.T, (ChanStats*)ctx->cs.p, (float*)ctx->sigma.p);
+    k_mel_stats<<<d.n, 128, 0, st>>>(cp, cb, ctx->sh ? ctx->sh->T_glob : d.T, (ChanStats*)ctx->cs.p, (float*)ctx->sigma.p);
     ctx->launches++;
     AW_LAUNCH_CHECK();
     prof_mark(ctx, st, "p0");
-    aw_launch(ctx, k_p0<AT>, dim3(g2), dim3(128), 0, st, (float*)ctx->M.p, d.T, d.Tp, d.Tp_pad, (ChanStats*)ctx->cs.p,
+    k_p0<AT><<<g2, 128, 0, st>>>((float*)ctx->M.p, d.T, d.Tp, d.Tp_pad, (ChanStats*)ctx->cs.p,
                                  (float*)ctx->sigma.p, (AT*)ctx->act[0].p, tf);
     ctx->launches++;
     AW_LAUNCH_CHECK();
@@ -1105,17 +1010,6 @@ static int net_forward(aw_ctx* ctx, const Dims& d, const Acc& acc, const SparseM
     // output, so it runs twice -- column sums only, then again with InstanceNorm + LeakyReLU applied in
     // the epilogue -- and the raw H1 never exists (exact fp32 mode keeps the one-pass form)
     const bool two_pass = l == 0 && ctx->prec != AW_PREC_FP32 && ctx->two_pass;
-    const int fuse = two_pass || ctx->prec == AW_PREC_FP32 ? 0 : fuse_form(ctx, 1, d.n, d.tiles, d.rows, cout, cin, (int)sizeof(AT));
-    if (fuse) {
-      // InstanceNorm + LeakyReLU inside the GEMM: H never exists, no finalize / apply pass
-      if constexpr (sizeof(AT) == 2) {
-        ep.tiles_per_clip = d.tiles; ep.Tp = d.Tp; ep.stat_out = (float*)ctx->stat[l + 1].p;
-        if (fuse == 2 ? launch_tc_fused<AT, AT, EPI_FWD_FUSE, 2>(ctx, ctx->tm_act[B][l], ModeOf<AT>::wP(ctx, l), d.rows, cout, cin, ep, d.n, st)
-                      : launch_tc_fused<AT, AT, EPI_FWD_FUSE, 1>(ctx, ctx->tm_act[B][l], mw, d.rows, cout, cin, ep, d.n, st))
-          return 1;
-      }
-      continue;
-    }
     if (two_pass) {
       if (launch_tc<AT, AT, 256, EPI_FWD_STATS>(ctx, ctx->tm_act[B][l], mw, d.rows, cout, cin, ep, st)) return 1;
     } else if (ctx->prec != AW_PREC_FP32 && pair_ok(ctx, d.rows, cout, cin, (int)sizeof(AT))) {
@@ -1129,11 +1023,11 @@ static int net_forward(aw_ctx* ctx, const Dims& d, const Acc& acc, const SparseM
       if (sh_finalize<false>(ctx, cout, d.tiles, (float*)ctx->stat[l + 1].p, st)) return 1;
     } else {
       if (d.tiles <= 16)
-        aw_launch(ctx, k_finalize_small<0>, dim3((cout + 255) / 256, d.n), dim3(256), 0, st, (float*)ctx->part.p, cout, d.tiles, cout,
+        k_finalize_small<0><<<dim3((cout + 255) / 256, d.n), 256, 0, st>>>((float*)ctx->part.p, cout, d.tiles, cout,
                                                                            d.Tp, (float*)ctx->stat[l + 1].p);
       else
-        aw_launch(ctx, k_finalize<0>, dim3(g), dim3(256), 0, st, (float*)ctx->part.p, cout, d.tiles, cout, d.Tp,
-                  (float*)ctx->stat[l + 1].p, nullptr);
+        k_finalize<0><<<g, 256, 0, st>>>((float*)ctx->part.p, cout, d.tiles, cout, d.Tp,
+                                         (float*)ctx->stat[l + 1].p, nullptr);
       ctx->launches++;
       AW_LAUNCH_CHECK();
     }
@@ -1146,7 +1040,7 @@ static int net_forward(aw_ctx* ctx, const Dims& d, const Acc& acc, const SparseM
     {
       const int rl = 128 / std::min(128, cout / Vec16<AT>::N);       // row lanes per block (narrow layers)
       dim3 gn((d.Tp_pad + AW_NORM_ROWS * rl - 1) / (AW_NORM_ROWS * rl), (cout / Vec16<AT>::N + 127) / 128, d.n);
-      aw_launch(ctx, k_norm_rows<AT, NORM_FWD>, dim3(gn), dim3(128), 0, st, (AT*)ctx->act[l + 1].p, nullptr, cout, d.Tp, d.Tp_pad,
+      k_norm_rows<AT, NORM_FWD><<<gn, 128, 0, st>>>((AT*)ctx->act[l + 1].p, nullptr, cout, d.Tp, d.Tp_pad,
                                                     (float*)ctx->stat[l + 1].p, nullptr, tf && l < 3);
     }
     ctx->launches++;
@@ -1183,17 +1077,6 @@ static int net_backward(aw_ctx* ctx, const Dims& d, const Acc& acc, const Sparse
     memset(&g64, 0, sizeof(g64));
     g64.part = (float*)ctx->part.p; g64.ldp = n; g64.ldo = n; g64.tiles_per_clip = d.tiles; g64.Tp = d.Tp;
     g64.stat = (float*)ctx->stat[l].p; g64.bstat = (float*)ctx->bstat.p;
-    const int fuse = two_pass || ctx->prec == AW_PREC_FP32 ? 0 : fuse_form(ctx, 2, d.n, d.tiles, d.rows, n, k, (int)sizeof(AT));
-    if (fuse) {
-      // LeakyReLU' + InstanceNorm adjoint inside the GEMM: dHhat never exists, no finalize / apply pass
-      if constexpr (sizeof(AT) == 2) {
-        ep.tiles_per_clip = d.tiles; ep.Tp = d.Tp; ep.stat = (float*)ctx->stat[l].p;
-        if (fuse == 2 ? launch_tc_fused<AT, AT, EPI_BWD_FUSE, 2>(ctx, *steps[s].ma, ModeOf<AT>::wtP(ctx, l), d.rows, n, k, ep, d.n, st)
-                      : launch_tc_fused<AT, AT, EPI_BWD_FUSE, 1>(ctx, *steps[s].ma, mw, d.rows, n, k, ep, d.n, st))
-          return 1;
-      }
-      continue;
-    }
     if (stream64) {
       if constexpr (sizeof(AT) == 2) {
         if (launch_bwd64<AT, EPI_BWD_STATS>(ctx, *steps[s].ma, ModeOf<AT>::wtP(ctx, l), ctx->tm_act[B][l], ctx->tm_ga1024[B],
@@ -1211,11 +1094,11 @@ static int net_backward(aw_ctx* ctx, const Dims& d, const Acc& acc, const Sparse
       if (sh_finalize<true>(ctx, n, d.tiles, (float*)ctx->bstat.p, st)) return 1;
     } else {
       if (d.tiles <= 16)
-        aw_launch(ctx, k_finalize_small<1>, dim3((n + 255) / 256, d.n), dim3(256), 0, st, (float*)ctx->part.p, n, d.tiles, n, d.Tp,
+        k_finalize_small<1><<<dim3((n + 255) / 256, d.n), 256, 0, st>>>((float*)ctx->part.p, n, d.tiles, n, d.Tp,
                                                                         (float*)ctx->bstat.p);
       else
-        aw_launch(ctx, k_finalize<1>, dim3(g), dim3(256), 0, st, (float*)ctx->part.p, n, d.tiles, n, d.Tp,
-                  (float*)ctx->bstat.p, nullptr);
+        k_finalize<1><<<g, 256, 0, st>>>((float*)ctx->part.p, n, d.tiles, n, d.Tp,
+                                         (float*)ctx->bstat.p, nullptr);
       ctx->launches++;
       AW_LAUNCH_CHECK();
     }
@@ -1237,7 +1120,7 @@ static int net_backward(aw_ctx* ctx, const Dims& d, const Acc& acc, const Sparse
     {
       const int rl = 128 / std::min(128, n / Vec16<AT>::N);
       dim3 gn((d.Tp_pad + AW_NORM_ROWS * rl - 1) / (AW_NORM_ROWS * rl), (n / Vec16<AT>::N + 127) / 128, d.n);
-      aw_launch(ctx, k_norm_rows<AT, NORM_BWD>, dim3(gn), dim3(128), 0, st, steps[s].out, (AT*)ctx->act[l].p, n, d.Tp, d.Tp_pad,
+      k_norm_rows<AT, NORM_BWD><<<gn, 128, 0, st>>>(steps[s].out, (AT*)ctx->act[l].p, n, d.Tp, d.Tp_pad,
                                                     (float*)ctx->stat[l].p, (float*)ctx->bstat.p, tf);
     }
     ctx->launches++;
@@ -1261,7 +1144,7 @@ static int net_backward(aw_ctx* ctx, const Dims& d, const Acc& acc, const Sparse
   }
   dim3 g1((2 * d.Tp + AW_P0B_FRAMES - 1) / AW_P0B_FRAMES, d.n);
   prof_mark(ctx, st, "p0_bwd_reduce");
-  aw_launch(ctx, k_p0_bwd_reduce, dim3(g1), dim3(128), 0, st, (float*)ctx->dp0.p, (float*)ctx->M.p, d.T, d.Tp, d.Tp_pad,
+  k_p0_bwd_reduce<<<g1, 128, 0, st>>>((float*)ctx->dp0.p, (float*)ctx->M.p, d.T, d.Tp, d.Tp_pad,
                                       (ChanStats*)ctx->cs.p, acc.bpart, (const float*)ctx->gsc.p);
   ctx->launches++;
   AW_LAUNCH_CHECK();
@@ -1274,12 +1157,12 @@ static int net_backward(aw_ctx* ctx, const Dims& d, const Acc& acc, const Sparse
     bb = 1;
   } else if (reduce_if_long(ctx, ctx->red_b, bp, bb, d.n, 2 * AW_NMEL, st)) return 1;
   prof_mark(ctx, st, "p0_bwd_coef");
-  aw_launch(ctx, k_p0_bwd_coef, dim3(d.n), dim3(128), 0, st, bp, bb, ctx->sh ? ctx->sh->T_glob : d.T, (ChanStats*)ctx->cs.p, (float*)ctx->sigma.p,
+  k_p0_bwd_coef<<<d.n, 128, 0, st>>>(bp, bb, ctx->sh ? ctx->sh->T_glob : d.T, (ChanStats*)ctx->cs.p, (float*)ctx->sigma.p,
                                      (P0BwdCoef*)ctx->p0coef.p, (P0BwdScal*)ctx->p0scal.p);
   ctx->launches++;
   AW_LAUNCH_CHECK();
   prof_mark(ctx, st, "p0_bwd_apply");
-  aw_launch(ctx, k_p0_bwd_apply, dim3(g2), dim3(128), 0, st, (float*)ctx->dp0.p, (float*)ctx->M.p, d.T, d.Tp, d.Tp_pad,
+  k_p0_bwd_apply<<<g2, 128, 0, st>>>((float*)ctx->dp0.p, (float*)ctx->M.p, d.T, d.Tp, d.Tp_pad,
                                      (ChanStats*)ctx->cs.p, (P0BwdCoef*)ctx->p0coef.p,
                                      (P0BwdScal*)ctx->p0scal.p, sm, d.nb, own_frames(ctx, (float*)ctx->dA.p, d.nb),
                                      euler_s2 ? (const float*)own_frames(ctx, (float*)ctx->mag.p, d.nb) : nullptr, acc.s2_part,
@@ -1306,18 +1189,18 @@ static int run_head(aw_ctx* ctx, const Dims& d, const float* pattern, float* val
   h.hpart = (double*)ctx->hpart.p;
   h.hcoef = (float*)ctx->hcoef.p;
   prof_mark(ctx, st, "head");
-  aw_launch(ctx, k_head_partial<AT>, dim3(d.tiles, d.n), dim3(256), 0, st, h);
+  k_head_partial<AT><<<dim3(d.tiles, d.n), 256, 0, st>>>(h);
   if (ctx->sh) {
     if (sh_reduce_sum(ctx, ctx->red_a, h.hpart, d.tiles, 64 * 3, st)) return 1;
     HeadArgs<AT> hf = h;
     hf.hpart = const_cast<double*>(sh_red(ctx));
-    aw_launch(ctx, k_head_final<AT>, dim3(d.n), dim3(64), 0, st, hf, 1);
+    k_head_final<AT><<<d.n, 64, 0, st>>>(hf, 1);
   } else {
-    aw_launch(ctx, k_head_final<AT>, dim3(d.n), dim3(64), 0, st, h, d.tiles);
+    k_head_final<AT><<<d.n, 64, 0, st>>>(h, d.tiles);
   }
   ctx->launches += 2;
   if (backward && pattern) {
-    aw_launch(ctx, k_head_seed<AT>, dim3(d.tiles, d.n), dim3(256), 0, st, h);
+    k_head_seed<AT><<<dim3(d.tiles, d.n), 256, 0, st>>>(h);
     ctx->launches++;
   }
   AW_LAUNCH_CHECK();
@@ -1384,7 +1267,7 @@ static int launch_spec_k(aw_ctx* ctx, const Dims& d, SpecArgs& a, cudaStream_t s
   const int items = a.edge_mode ? a.n_clips * 2 : a.n_clips * a.tiles;
   const int grid = std::min(items, 2 * ctx->num_sms);
   prof_mark(ctx, st, a.edge_mode ? (MODE == SPEC_FWD ? "spec_edge_fwd" : "spec_edge_bwd") : (MODE == SPEC_FWD ? "spec_fwd" : "spec_bwd"));
-  aw_launch(ctx, k_spec<MODE, K2LO, K2HI>, dim3(grid), dim3(32 * AW_SP_WARPS), AW_SP_SMEM, st, a);
+  k_spec<MODE, K2LO, K2HI><<<grid, 32 * AW_SP_WARPS, AW_SP_SMEM, st>>>(a);
   ctx->launches++;
   AW_LAUNCH_CHECK();
   return 0;
@@ -1417,7 +1300,7 @@ static int launch_peak(aw_ctx* ctx, const float* x, int64_t stride, int n, int n
 }
 static int begin_pass(aw_ctx* ctx, int n, int* it, cudaStream_t st, unsigned* dmax = nullptr) {
   prof_mark(ctx, st, "iter_begin");
-  aw_launch(ctx, k_iter_begin, dim3((n + 255) / 256), dim3(256), 0, st, (unsigned long long*)ctx->accum.p, n, it, dmax);
+  k_iter_begin<<<(n + 255) / 256, 256, 0, st>>>((unsigned long long*)ctx->accum.p, n, it, dmax);
   ctx->launches++;
   AW_LAUNCH_CHECK();
   return 0;
@@ -1658,8 +1541,8 @@ static int tc_backward(aw_ctx* ctx, const Dims& d, int* itc, cudaStream_t st, in
     ctx->launches++;
   }
   prof_mark(ctx, st, "tc_dsprep");
-  aw_launch(ctx, k_tc_dsprep, dim3((d.T + AW_TC_FR - 1) / AW_TC_FR, d.n), dim3(256), 0, st, (const float*)ctx->dA.p, (const float2*)ctx->ph_q.p, d.T, d.nb,
-                                               (unsigned*)ctx->tc_dmax.p, itc, d.n, (__half*)ctx->tc_dS.p);
+  k_tc_dsprep<<<dim3((d.T + AW_TC_FR - 1) / AW_TC_FR, d.n), 256, 0, st>>>((const float*)ctx->dA.p, (const float2*)ctx->ph_q.p, d.T, d.nb,
+                                                                          (unsigned*)ctx->tc_dmax.p, itc, d.n, (__half*)ctx->tc_dS.p);
   ctx->launches++;
   AW_LAUNCH_CHECK();
   EpiArgsT<float> ep = tc_epi(d);
@@ -1688,7 +1571,7 @@ static int tc_backward(aw_ctx* ctx, const Dims& d, int* itc, cudaStream_t st, in
   u.X = (__half*)ctx->tc_X.p;
   u.nonfinite = nonfinite;
   prof_mark(ctx, st, "tc_update");
-  aw_launch(ctx, k_tc_update, dim3((d.T + AW_TC_FR - 1) / AW_TC_FR, d.n), dim3(256), 0, st, u);
+  k_tc_update<<<dim3((d.T + AW_TC_FR - 1) / AW_TC_FR, d.n), 256, 0, st>>>(u);
   ctx->launches++;
   AW_LAUNCH_CHECK();
   return 0;
@@ -1806,12 +1689,6 @@ extern "C" int aw_embed_batch(aw_ctx* ctx, const float* d_audio, int n_clips, in
 
     // ---- optimisation loop (multibit_embedder.py:95-122)
     nvtxRangePushA("embed:nadam_loop");
-    // programmatic dependent launch inside the loop (opt-in, AW_B200_PDL=1): every kernel is scheduled while its
-    // predecessor drains and waits in pdl_wait() for its completion.  Measured: 256 clips 5.1-5.3 ms per
-    // iteration against 4.84-4.91 without (the early-resident successors take registers and issue slots from
-    // the running kernel), one clip 0.24-0.27 ms either way -- hence off by default
-    struct PdlScope { aw_ctx* c; ~PdlScope() { c->pdl = false; } } pdl_scope_{ctx};
-    ctx->pdl = ctx->pdl_ok && !ctx->prof_on;
     auto iteration = [&](bool first) -> int {
       // fused spectral passes (spec.cuh): y and dpad never leave shared memory
       if (begin_pass(ctx, dw.n, itc, st)) return 1;
@@ -1847,7 +1724,7 @@ extern "C" int aw_embed_batch(aw_ctx* ctx, const float* d_audio, int n_clips, in
       if (reduce_if_long(ctx, ctx->red_c, sp2, sb2, dw.n, 1, st)) return 1;
       if (sb2 > 512 && reduce_if_long(ctx, ctx->red_a, sp2, sb2, dw.n, 1, st)) return 1;   // 1 h: 38 760 -> 606 -> 10
       prof_mark(ctx, st, "clip_scalars");
-      aw_launch(ctx, k_clip_scalars, dim3((dw.n + 127) / 128), dim3(128), 0, st, acc.peak_y, sp2, sb2, dw.n, (ClipScal*)ctx->scal.p, 0,
+      k_clip_scalars<<<(dw.n + 127) / 128, 128, 0, st>>>(acc.peak_y, sp2, sb2, dw.n, (ClipScal*)ctx->scal.p, 0,
                                                          tc ? (unsigned*)ctx->tc_dmax.p : nullptr, itc);
       ctx->launches++;
       AW_LAUNCH_CHECK();
@@ -1898,7 +1775,6 @@ extern "C" int aw_embed_batch(aw_ctx* ctx, const float* d_audio, int n_clips, in
       for (int it = 0; it < iters; ++it)
         if (iteration(it == 0)) return 1;
     }
-    ctx->pdl = false;
     nvtxRangePop();
     // ---- final synthesis from the best coefficients (multibit_embedder.py:173-192)
     nvtxRangePushA("embed:final_synthesis");
@@ -2098,8 +1974,8 @@ extern "C" int aw_embed_sharded(aw_ctx* ctx, const float* d_segment, int seg_sam
     if (rc) return 1;
     if (sh_reduce_sum(ctx, ctx->red_c, acc.s2_part, p0a_blocks(dn), 1, st)) return 1;   // Euler sum over the clip
     prof_mark(ctx, st, "clip_scalars");
-    aw_launch(ctx, k_clip_scalars, dim3(1), dim3(128), 0, st, acc.peak_y, sh_red(ctx), 1, 1, (ClipScal*)ctx->scal.p, n_base,
-              nullptr, nullptr);
+    k_clip_scalars<<<1, 128, 0, st>>>(acc.peak_y, sh_red(ctx), 1, 1, (ClipScal*)ctx->scal.p, n_base,
+                                      nullptr, nullptr);
     ctx->launches++;
     AW_LAUNCH_CHECK();
     if (sh_halo_exchange(ctx, (float*)ctx->dA.p, ds.nb, st)) return 1;   // spectral gradient of the halo frames

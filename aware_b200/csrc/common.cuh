@@ -106,14 +106,6 @@ __device__ __forceinline__ unsigned peak_index(unsigned long long p) {
 
 __device__ __forceinline__ float leaky(float x) { return x > 0.f ? x : AW_LEAKY * x; }
 
-// Programmatic dependent launch (PDL): inside the optimisation loop every kernel is launched with
-// programmatic stream serialisation, so it can be scheduled while its predecessor drains.  pdl_wait() blocks
-// until the predecessor grid has completed and its writes are visible (a no-op for an ordinary launch);
-// pdl_trigger() lets the successor be scheduled early.  Every kernel of the loop calls both first thing.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_enter() { pdl_trigger(); pdl_wait(); }
-
 // round-to-nearest TF32 (keeps the value in a float container)
 __device__ __forceinline__ float to_tf32(float x) {
   uint32_t r;

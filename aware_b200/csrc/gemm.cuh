@@ -28,17 +28,11 @@ namespace aw {
 // iSTFT as a GEMM whose epilogue adds the constant out-of-band waveform and reduces max|y| (nothing is
 // stored), and the band-limited STFT o iSTFT composite whose epilogue adds the constant out-of-band
 // spectrum and writes |S| and S/|S|.
-// EPI_FWD_FUSE / EPI_BWD_FUSE: InstanceNorm (+ LeakyReLU) / its adjoint applied INSIDE the K >= 512 GEMMs.  The
-// accumulator tile stays in TMEM while the CTAs that hold the other row tiles of the same clip and column panel
-// publish their column sums (global partials + one counter per (clip, panel)); the epilogue then reads the
-// accumulator a second time and stores the normalised tile, so the raw H / dHhat never exists in HBM and the
-// stand-alone finalize + apply passes disappear (see the tile order in gemm_tile_rc).
 enum { EPI_PLAIN = 0, EPI_FWD = 1, EPI_BWD = 2, EPI_FWD_STATS = 3, EPI_FWD_APPLY = 4, EPI_BWD_STATS = 5,
-       EPI_BWD_APPLY = 6, EPI_PEAK = 7, EPI_SPEC = 8, EPI_FWD_FUSE = 9, EPI_BWD_FUSE = 10 };
-__host__ __device__ constexpr bool epi_fused(int e) { return e == EPI_FWD_FUSE || e == EPI_BWD_FUSE; }
-__host__ __device__ constexpr bool epi_is_bwd(int e) { return e == EPI_BWD || e == EPI_BWD_STATS || e == EPI_BWD_APPLY || e == EPI_BWD_FUSE; }
-__host__ __device__ constexpr bool epi_is_fwd(int e) { return e == EPI_FWD || e == EPI_FWD_STATS || e == EPI_FWD_APPLY || e == EPI_FWD_FUSE; }
-__host__ __device__ constexpr bool epi_has_stats(int e) { return e == EPI_FWD || e == EPI_BWD || e == EPI_FWD_STATS || e == EPI_BWD_STATS || epi_fused(e); }
+       EPI_BWD_APPLY = 6, EPI_PEAK = 7, EPI_SPEC = 8 };
+__host__ __device__ constexpr bool epi_is_bwd(int e) { return e == EPI_BWD || e == EPI_BWD_STATS || e == EPI_BWD_APPLY; }
+__host__ __device__ constexpr bool epi_is_fwd(int e) { return e == EPI_FWD || e == EPI_FWD_STATS || e == EPI_FWD_APPLY; }
+__host__ __device__ constexpr bool epi_has_stats(int e) { return e == EPI_FWD || e == EPI_BWD || e == EPI_FWD_STATS || e == EPI_BWD_STATS; }
 __host__ __device__ constexpr bool epi_stores(int e) { return e != EPI_FWD_STATS && e != EPI_BWD_STATS && e != EPI_PEAK && e != EPI_SPEC; }
 __host__ __device__ constexpr bool epi_applies(int e) { return e == EPI_FWD_APPLY || e == EPI_BWD_APPLY; }
 
@@ -260,15 +254,9 @@ __device__ __forceinline__ float warp_colsum32(float (&v)[32], int lane) {
 // Epilogues that hold an operand ring in registers run the three-warpgroup layout; the others keep the
 // compact one (warp 0 TMA, warp 1 MMA, warps 2..9 epilogue; 320 threads, no register hand-over).
 __host__ __device__ constexpr bool gemm_big_epi(int e) {
-  return e == EPI_PEAK || e == EPI_SPEC || e == EPI_BWD || e == EPI_BWD_STATS || e == EPI_BWD_FUSE;
+  return e == EPI_PEAK || e == EPI_SPEC || e == EPI_BWD || e == EPI_BWD_STATS;
 }
-// EPI_FWD_FUSE on CTA pairs runs TWO sets of eight epilogue warps, one per TMEM accumulator buffer (set s drains
-// the tiles of rounds s, s + 2, ...): while one set waits for the other CTAs' column sums, the other set reads /
-// normalises / stores its own tile, and four epilogue warps per scheduler instead of two hide each other's latencies.
-__host__ __device__ constexpr int gemm_epi_sets(int e, int cg) { return e == EPI_FWD_FUSE && cg == 2 ? 2 : 1; }
-__host__ __device__ constexpr int gemm_threads(int e, int cg = 1) {
-  return gemm_big_epi(e) ? AW_GEMM_THREADS : 64 + 256 * gemm_epi_sets(e, cg);
-}
+__host__ __device__ constexpr int gemm_threads(int e) { return gemm_big_epi(e) ? AW_GEMM_THREADS : 320; }
 #define AW_GEMM_REGS_LIGHT 56
 #define AW_GEMM_REGS_EPI 224
 
@@ -378,12 +366,6 @@ struct EpiArgsT {
   int tiles_per_clip;    // 128-row tiles per clip (Tp_pad / 128)
   int Tp;                // valid pooled frames per clip: rows beyond are written as 0
   int round_tf32;
-  // EPI_*_FUSE: one arrival counter per (clip, column panel), monotonically increasing (every launch adds
-  // tiles_per_clip to each: no reset between launches); tiles of a group = consecutive tile indices that run
-  // concurrently (gemm_tile_rc); FWD_FUSE also writes the finished (mean, rstd) for the backward pass
-  unsigned* fuse_cnt;
-  int fuse_gs;
-  float* stat_out;
   // Toeplitz A operand (spectral path): map_a is the plain 2-D map of an array of frame rows
   // [rows + pad][P]; k-block kb of GEMM row r is elements (kb % (P/BK)) * BK .. of frame row
   // r + kb / (P/BK), i.e. GEMM row r is the concatenation of K / P consecutive frame rows.  0 = ordinary.
@@ -412,43 +394,25 @@ __host__ __device__ constexpr int gemm_stages() { return BN == 256 ? 3 : AW_GEMM
 template <int BN>
 __host__ __device__ constexpr int gemm_tmem_cols() { return BN == 192 ? 512 : 2 * BN; }   // power of two >= 2 BN
 // CTA pair: every CTA stages its own 128 rows of A and HALF of the B tile, so a stage is a third smaller
-template <int BN, int EPI = EPI_PLAIN>
-__host__ __device__ constexpr int gemm_stages_pair() { return gemm_epi_sets(EPI, 2) == 2 ? 4 : (BN == 256 ? 5 : 6); }
-template <int BN, int EPI = EPI_PLAIN>
+template <int BN>
+__host__ __device__ constexpr int gemm_stages_pair() { return BN == 256 ? 5 : 6; }
+template <int BN>
 constexpr int gemm_tc_smem_pair() {
-  return gemm_stages_pair<BN, EPI>() * (128 * 128 + BN / 2 * 128) + 1024 + 256 + 2 * 2 * 4 * BN * 4 +
-         gemm_epi_sets(EPI, 2) * (8 * AW_EPI_STAGE_WORDS * 4 + 3 * BN * 4);
+  return gemm_stages_pair<BN>() * (128 * 128 + BN / 2 * 128) + 1024 + 256 + 2 * 2 * 4 * BN * 4 +
+         8 * AW_EPI_STAGE_WORDS * 4;
 }
 template <int BN>
 constexpr int gemm_tc_smem() {
   return gemm_stages<BN>() * (128 * 128 + BN * 128) + 1024 /*align*/ + 256 /*barriers*/ +
          2 * 2 * 4 * BN * 4 /*double-buffered column partials*/ +
-         8 * AW_EPI_STAGE_WORDS * 4 /*per-warp epilogue transpose tiles*/ +
-         3 * BN * 4 /*EPI_*_FUSE: the panel's column statistics*/;
+         8 * AW_EPI_STAGE_WORDS * 4 /*per-warp epilogue transpose tiles*/;
 }
 
-// Tile index -> (128-row tile, column tile).  Ordinary epilogues: column tile fastest.  EPI_*_FUSE: the `gs`
-// (pair-)tiles of a GROUP -- all row tiles of one clip (CTA pairs, odd tile count: of two clips) for ONE column
-// panel -- are consecutive tile indices, and the grid is a multiple of `gs`, so a group's tiles are processed in
-// the same round by `gs` consecutive CTAs (pairs): they finish their accumulators together and each waits only
-// for peers that are resident and at the same tile.  Consecutive groups walk the column panels of the same
-// clips, so concurrently running CTAs still share A row tiles in L2.
-template <int EPI, int CG>
-__device__ __forceinline__ void gemm_tile_rc(int tile, int n_col_tiles, int gs, uint32_t rank, int& row_tile,
-                                             int& col_tile) {
-  if (epi_fused(EPI)) {
-    const int g = tile / gs, j = tile - g * gs;
-    row_tile = ((g / n_col_tiles) * gs + j) * CG + (int)rank;
-    col_tile = g % n_col_tiles;
-  } else {
-    row_tile = (tile / n_col_tiles) * CG + (int)rank;
-    col_tile = tile % n_col_tiles;
-  }
-}
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
+// Tile index -> (128-row tile, column tile), column tile fastest
+template <int CG>
+__device__ __forceinline__ void gemm_tile_rc(int tile, int n_col_tiles, uint32_t rank, int& row_tile, int& col_tile) {
+  row_tile = (tile / n_col_tiles) * CG + (int)rank;
+  col_tile = tile % n_col_tiles;
 }
 
 // Persistent tcgen05 GEMM.  grid = min(#tiles, #SMs); every CTA walks tiles
@@ -463,7 +427,6 @@ __device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
 template <typename T, typename OT, int BN, int EPI, int CG>
 __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUtensorMap& map_b,
                                              int K, int n_row_tiles, int n_col_tiles, const EpiArgsT<OT>& ep) {
-  pdl_trigger();                                     // the successor may be scheduled while this grid runs
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment by POINTER arithmetic on the __shared__ array: a round trip through uintptr_t made
   // the compiler forget the address space, every epilogue staging access became a generic LD.E / ST.E on the
@@ -475,8 +438,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
 #endif
   constexpr int BK = GemmElem<T>::BK;
-  constexpr int NSTAGE = CG == 2 ? gemm_stages_pair<BN, EPI>() : gemm_stages<BN>();
-  constexpr int NSETS = gemm_epi_sets(EPI, CG);
+  constexpr int NSTAGE = CG == 2 ? gemm_stages_pair<BN>() : gemm_stages<BN>();
   constexpr int A_BYTES = 128 * 128, B_BYTES = BN / CG * 128, STAGE = A_BYTES + B_BYTES;
   const uint32_t rank = CG == 2 ? cluster_ctarank() : 0u;
   const int unit = CG == 2 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;          // tile walker: CTA or CTA pair
@@ -489,9 +451,6 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
   float* s_part = reinterpret_cast<float*>(smem + NSTAGE * STAGE + 256);  // [2][2][4][BN]
   float* s_stage = s_part + 2 * 2 * 4 * BN;                                       // [8 warps][32][36]
-  float* s_fs = s_stage + 8 * NSETS * AW_EPI_STAGE_WORDS;                         // [NSETS][3][BN] EPI_*_FUSE statistics
-  constexpr bool FUSE = epi_fused(EPI);
-  constexpr int NPASS = FUSE ? 2 : 1;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nkb = K / BK;
@@ -530,9 +489,6 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
   if (CG == 2) cluster_sync_all();                   // both CTAs' barriers exist before any remote arrive
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // barriers, TMEM and descriptors are set up: everything above overlapped the predecessor's tail (PDL);
-  // from here on its output is read
-  pdl_wait();
   const uint32_t leader_full = CG == 2 ? mapa_u32(smem_u32(full), 0) : 0u;
   const uint32_t leader_tempty = CG == 2 ? mapa_u32(smem_u32(tempty), 0) : 0u;
   // register hand-over between warpgroups (see AW_GEMM_THREADS); each setmaxnreg sits at the head of the
@@ -548,7 +504,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
       uint32_t ph = 0;
       for (int tile = unit; tile < n_tiles; tile += n_units) {
         int rt_, ct_;
-        gemm_tile_rc<EPI, CG>(tile, n_col_tiles, ep.fuse_gs, rank, rt_, ct_);
+        gemm_tile_rc<CG>(tile, n_col_tiles, rank, rt_, ct_);
         const int row0 = rt_ * 128, n0 = ct_ * BN;
         for (int kb = 0; kb < nkb; ++kb) {
           mbar_wait(empty + s, ph ^ 1);
@@ -611,9 +567,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
   } else {
     // -------------------------------- epilogue --------------------------------
     if (BIG) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(AW_GEMM_REGS_EPI));
-    const int e16 = warp - EW0;
-    const int set = NSETS == 2 ? e16 >> 3 : 0;      // epilogue warp set = TMEM accumulator buffer it drains
-    const int e = e16 & 7;
+    const int e = warp - EW0;
     const int q = warp & 3;                         // TMEM lane quarter this warp may access
     const int half = e >> 2;                        // which half of the BN columns
     constexpr int CHUNKS = BN / 64;                 // 32-column chunks per warp
@@ -622,7 +576,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
     // two-slot register ring, and the loads of chunk c + 1 are issued right after chunk c's registers have
     // been consumed.  (Issuing further ahead does not help: the hardware scoreboards are few, the wait for
     // chunk c's data then also waits for the younger loads queued on the same scoreboard -- ncu source view.)
-    constexpr bool PF = (EPI == EPI_BWD || EPI == EPI_BWD_STATS || EPI == EPI_BWD_FUSE) && CHUNKS == 4;
+    constexpr bool PF = (EPI == EPI_BWD || EPI == EPI_BWD_STATS) && CHUNKS == 4;
     constexpr bool SPF = EPI == EPI_FWD_APPLY && CHUNKS == 4;
     constexpr int NB = 2;
     ActRaw<OT> gr[PF ? NB : 1][8];
@@ -630,12 +584,12 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
     const int sr_ = lane >> 3, cg_ = (lane & 7) * 4;
     auto act_tile_base = [&](int tile_) -> const OT* {
       int rt, ct;
-      gemm_tile_rc<EPI, CG>(tile_, n_col_tiles, ep.fuse_gs, rank, rt, ct);
+      gemm_tile_rc<CG>(tile_, n_col_tiles, rank, rt, ct);
       return ep.act + (long long)(rt * 128 + q * 32 + sr_) * ep.ldo + ct * BN + half * (BN / 2) + cg_;
     };
     auto stat_tile_base = [&](int tile_) -> long long {
       int rt, ct;
-      gemm_tile_rc<EPI, CG>(tile_, n_col_tiles, ep.fuse_gs, rank, rt, ct);
+      gemm_tile_rc<CG>(tile_, n_col_tiles, rank, rt, ct);
       return ((long long)(rt / ep.tiles_per_clip) * ep.ldo + ct * BN + half * (BN / 2) + cg_) * 2;
     };
     auto stat_load = [&](long long sb, float4 (&dst)[4]) {
@@ -654,21 +608,20 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
       }
       if (SPF) stat_load(stat_tile_base(unit), stq[0]);
     }
-    int it = set;
-    for (int tile = unit + set * n_units; tile < n_tiles; tile += NSETS * n_units, it += NSETS) {
+    int it = 0;
+    for (int tile = unit; tile < n_tiles; tile += n_units, ++it) {
       const int ab = it & 1;
       int row_tile, col_tile;
-      gemm_tile_rc<EPI, CG>(tile, n_col_tiles, ep.fuse_gs, rank, row_tile, col_tile);
+      gemm_tile_rc<CG>(tile, n_col_tiles, rank, row_tile, col_tile);
       const int n0 = col_tile * BN;
-      const bool has_next = tile + NSETS * n_units < n_tiles;
-      const OT* abase_next = PF && has_next ? act_tile_base(tile + NSETS * n_units) : nullptr;
-      const long long sbase_next = SPF && has_next ? stat_tile_base(tile + NSETS * n_units) : 0;
+      const bool has_next = tile + n_units < n_tiles;
+      const OT* abase_next = PF && has_next ? act_tile_base(tile + n_units) : nullptr;
+      const long long sbase_next = SPF && has_next ? stat_tile_base(tile + n_units) : 0;
       // Global traffic goes through a per-warp 32 x 32 transpose tile: TMEM hands every lane
       // one ROW (32 columns in registers), but a warp-wide access is only coalesced when
       // adjacent lanes touch adjacent columns.  Staged, one 16-byte instruction covers 4 rows
       // x 128 contiguous bytes (4 wavefronts) instead of 32 rows x 16 bytes (32 wavefronts).
-      float* s_st = s_stage + e16 * AW_EPI_STAGE_WORDS;
-      float* s_fs_set = s_fs + set * 3 * BN;
+      float* s_st = s_stage + e * AW_EPI_STAGE_WORDS;
       const int sr = lane >> 3, cg = (lane & 7) * 4;  // staged access: row 4 i + sr, columns cg .. cg+3
       const long long grow = (long long)(row_tile * 128 + q * 32 + sr) * ep.ldo + n0 + half * (BN / 2) + cg;
       OT* obase = epi_stores(EPI) ? ep.out + grow : nullptr;
@@ -706,8 +659,8 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
         }
       }
       // *_APPLY: this tile's clip, its first row inside the clip, and the statistics base
-      const int clip_ = epi_applies(EPI) || FUSE ? row_tile / ep.tiles_per_clip : 0;
-      const int jrow0 = epi_applies(EPI) || FUSE ? (row_tile - clip_ * ep.tiles_per_clip) * 128 + q * 32 + sr : 0;
+      const int clip_ = epi_applies(EPI) ? row_tile / ep.tiles_per_clip : 0;
+      const int jrow0 = epi_applies(EPI) ? (row_tile - clip_ * ep.tiles_per_clip) * 128 + q * 32 + sr : 0;
       const long long sbase = epi_applies(EPI) ? ((long long)clip_ * ep.ldo + n0 + half * (BN / 2) + cg) * 2 : 0;
       if (epi_is_bwd(EPI) && !PF) {                   // overlaps the wait for the accumulator
 #pragma unroll
@@ -739,12 +692,6 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
       if (EPI == EPI_SPEC) spec_load(0, so[0]);
       mbar_wait(tfull + ab, (it >> 1) & 1);
       tc_fence_after();
-      // EPI_*_FUSE reads the accumulator twice: pass 0 = column sums only, (exchange with the clip's other row
-      // tiles), pass 1 = apply + store; every other epilogue is the single pass 0
-#pragma unroll
-      for (int pass = 0; pass < NPASS; ++pass) {
-      const bool do_stats = epi_has_stats(EPI) && (!FUSE || pass == 0);
-      const bool do_store = epi_stores(EPI) && (!FUSE || pass == 1);
       // the TMEM load of chunk c+1 is in flight while chunk c is processed
       uint32_t vbuf[2][32];
       tc_ld32_async(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(ab * BN + half * (BN / 2)), vbuf[0]);
@@ -758,7 +705,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
           tc_wait_ld(v);
           if (c + 1 < CHUNKS)
             tc_ld32_async(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(ab * BN + c0 + 32), vbuf[(c + 1) & 1]);
-          if (c == CHUNKS - 1 && pass == NPASS - 1) {   // accumulator fully read: hand it back
+          if (c == CHUNKS - 1) {                    // accumulator fully read: hand it back
             tc_fence_before();
             __syncwarp();
             if (lane == 0) {
@@ -839,19 +786,6 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
         }
         float s1c[4] = {0.f, 0.f, 0.f, 0.f}, s2c[4] = {0.f, 0.f, 0.f, 0.f};
         float st_mu[4], st_rs[4], st_a1[4], st_a2[4];
-        if (FUSE && pass == 1) {                      // the panel's statistics, finished after pass 0
-          const float4 m4 = *reinterpret_cast<const float4*>(s_fs_set + c0 + cg);
-          const float4 r4 = *reinterpret_cast<const float4*>(s_fs_set + BN + c0 + cg);
-          if (EPI == EPI_FWD_FUSE) {
-            st_mu[0] = m4.x; st_mu[1] = m4.y; st_mu[2] = m4.z; st_mu[3] = m4.w;
-            st_rs[0] = r4.x; st_rs[1] = r4.y; st_rs[2] = r4.z; st_rs[3] = r4.w;
-          } else {
-            const float4 q4 = *reinterpret_cast<const float4*>(s_fs_set + 2 * BN + c0 + cg);
-            st_a1[0] = m4.x; st_a1[1] = m4.y; st_a1[2] = m4.z; st_a1[3] = m4.w;
-            st_a2[0] = r4.x; st_a2[1] = r4.y; st_a2[2] = r4.z; st_a2[3] = r4.w;
-            st_rs[0] = q4.x; st_rs[1] = q4.y; st_rs[2] = q4.z; st_rs[3] = q4.w;
-          }
-        }
         if (epi_applies(EPI)) {
           float4 s01, s23, b01 = make_float4(0.f, 0.f, 0.f, 0.f), b23 = b01;
           if (SPF) {
@@ -879,7 +813,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
         }
         // chunk c's operands are in plain registers now: queue the loads of the next chunk
         if (PF) {
-          const OT* src = c + 1 < CHUNKS ? abase + (c + 1) * 32 : (pass + 1 < NPASS ? abase : abase_next);
+          const OT* src = c + 1 < CHUNKS ? abase + (c + 1) * 32 : abase_next;
           if (src) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) act_ldraw(src + (long long)(4 * i) * ep.ldo, gr[PF ? ((c + 1) & 1) : 0][i]);
@@ -902,7 +836,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
               const bool pos = pv > 0.f;
               const float g = pos ? w[i][k] : AW_LEAKY * w[i][k];
               const float hh = pos ? pv : pv * (1.0f / AW_LEAKY);
-              if (EPI == EPI_BWD_APPLY || (EPI == EPI_BWD_FUSE && pass == 1)) {   // dH = rstd (dHhat - a1 - Hhat a2), pad rows 0 (k_norm_rows<BWD>)
+              if (EPI == EPI_BWD_APPLY) {               // dH = rstd (dHhat - a1 - Hhat a2), pad rows 0 (k_norm_rows<BWD>)
                 float o = st_rs[k] * (g - st_a1[k] - hh * st_a2[k]);
                 if (sizeof(OT) == 4 && ep.round_tf32) o = to_tf32(o);   // TF32 mode stores float activations
                 w[i][k] = jrow0 + 4 * i < ep.Tp ? o : 0.f;
@@ -917,7 +851,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
 #pragma unroll
             for (int i = 0; i < 8; ++i) act_ld4g(abase + (c + 1) * 32 + (long long)(4 * i) * ep.ldo, ga[i]);
           }
-        } else if (EPI == EPI_FWD_APPLY || (EPI == EPI_FWD_FUSE && pass == 1)) {   // P = LeakyReLU((H - mean) rstd), pad rows 0 (k_norm_rows<FWD>)
+        } else if (EPI == EPI_FWD_APPLY) {            // P = LeakyReLU((H - mean) rstd), pad rows 0 (k_norm_rows<FWD>)
 #pragma unroll
           for (int i = 0; i < 8; ++i)
 #pragma unroll
@@ -935,11 +869,11 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
               s2c[k] = fmaf(w[i][k], w[i][k], s2c[k]);
             }
         }
-        if (do_store) {
+        if (epi_stores(EPI)) {
 #pragma unroll
           for (int i = 0; i < 8; ++i) act_st4g(obase + c * 32 + (long long)(4 * i) * ep.ldo, w[i]);
         }
-        if (do_stats) {
+        if (epi_has_stats(EPI)) {
           // the 4 lanes that share (lane & 7) hold the same columns for different rows
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
@@ -961,9 +895,9 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
         if (lane == 0 && w0) atomicMax(ep.peak + sp_clip0, w0);
         if (lane == 0 && w1) atomicMax(ep.peak + sp_clip0 + 1, w1);
       }
-      if (do_stats) {
-        asm volatile("bar.sync %0, 256;" ::"r"(1 + set) : "memory");   // the 8 epilogue warps of this set
-        const int t = threadIdx.x - 32 * EW0 - 256 * set;             // 0..255
+      if (epi_has_stats(EPI)) {
+        asm volatile("bar.sync 1, 256;" ::: "memory");                // the 8 epilogue warps
+        const int t = threadIdx.x - 32 * EW0;                         // 0..255
         for (int cc = t; cc < BN; cc += 256) {
           float s1 = 0.f, s2 = 0.f;
 #pragma unroll
@@ -972,77 +906,10 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
             s2 += sp[(1 * 4 + w) * BN + cc];
           }
           float* p = ep.part + ((long long)row_tile * ep.ldp + n0 + cc) * 2;
-          if (FUSE) __stcg(reinterpret_cast<float2*>(p), make_float2(s1, s2));
-          else { p[0] = s1; p[1] = s2; }
-        }
-        if (FUSE) {
-          // publish this tile's column sums, wait for the clip's other row tiles of this panel (they are being
-          // finished right now by the neighbouring CTAs), then every CTA finalises the panel's statistics itself
-          // in k_finalize_small's float64 summation order
-          const int tpc = ep.tiles_per_clip;
-          asm volatile("bar.sync %0, 256;" ::"r"(1 + set) : "memory");
-          unsigned* cnt = ep.fuse_cnt + clip_ * n_col_tiles + col_tile;
-          if (t == 0) {
-            __threadfence();                               // cumulative: covers the set's stores ordered by the barrier
-            const unsigned old = atomicAdd(cnt, 1u);
-            const unsigned target = (old / (unsigned)tpc + 1u) * (unsigned)tpc;
-            uint32_t spins = 0;
-            while ((int)(ld_acquire_u32(cnt) - target) < 0) {
-              __nanosleep(20);
-              if (++spins > (1u << 25)) {
-                printf("aware_b200: fused InstanceNorm exchange timed out (block %d, tile %d)\n", blockIdx.x, tile);
-                __trap();
-              }
-            }
-          }
-          asm volatile("bar.sync %0, 256;" ::"r"(1 + set) : "memory");
-          for (int cc = t; cc < BN; cc += 256) {
-            const float* p0 = ep.part + ((long long)(clip_ * tpc) * ep.ldp + n0 + cc) * 2;
-            double s1 = 0.0, s2 = 0.0;
-            if (tpc <= 8) {
-              // one tile per slice: all loads in flight at once, summed in slice order
-              float2 pv[8];
-#pragma unroll
-              for (int tt = 0; tt < 8; ++tt)
-                pv[tt] = tt < tpc ? __ldcg(reinterpret_cast<const float2*>(p0 + (long long)tt * ep.ldp * 2)) : make_float2(0.f, 0.f);
-#pragma unroll
-              for (int tt = 0; tt < 8; ++tt) {
-                if (tt < tpc) {
-                  s1 = tt == 0 ? (double)pv[tt].x : s1 + (double)pv[tt].x;
-                  s2 = tt == 0 ? (double)pv[tt].y : s2 + (double)pv[tt].y;
-                }
-              }
-            } else {
-              for (int sl = 0; sl < 8; ++sl) {
-                double a1 = 0.0, a2 = 0.0;
-                for (int tt = sl; tt < tpc; tt += 8) {
-                  const float2 pv = __ldcg(reinterpret_cast<const float2*>(p0 + (long long)tt * ep.ldp * 2));
-                  a1 += pv.x;
-                  a2 += pv.y;
-                }
-                s1 = sl == 0 ? a1 : s1 + a1;
-                s2 = sl == 0 ? a2 : s2 + a2;
-              }
-            }
-            const long long so = ((long long)clip_ * ep.ldo + n0 + cc) * 2;
-            if (EPI == EPI_FWD_FUSE) {
-              const double mu = s1 / ep.Tp;
-              double var = s2 / ep.Tp - mu * mu;
-              if (var < 0.0) var = 0.0;
-              const float fmu = (float)mu, frs = (float)(1.0 / sqrt(var + AW_IN_EPS));
-              s_fs_set[cc] = fmu;
-              s_fs_set[BN + cc] = frs;
-              if (row_tile == clip_ * tpc) { ep.stat_out[so] = fmu; ep.stat_out[so + 1] = frs; }
-            } else {
-              s_fs_set[cc] = (float)(s1 / ep.Tp);
-              s_fs_set[BN + cc] = (float)(s2 / ep.Tp);
-              s_fs_set[2 * BN + cc] = __ldg(ep.stat + so + 1);
-            }
-          }
-          asm volatile("bar.sync %0, 256;" ::"r"(1 + set) : "memory");
+          p[0] = s1;
+          p[1] = s2;
         }
       }
-      }   // pass
     }
   }
   tc_fence_before();
@@ -1067,7 +934,7 @@ k_gemm_tc(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
 
 // CTA-pair form: map_b's box holds BN / 2 rows; n_row_tiles must be even; grid = 2 x #pairs
 template <typename T, typename OT, int BN, int EPI>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(gemm_threads(EPI, 2), 1)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(gemm_threads(EPI), 1)
 k_gemm_tc_pair(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                int K, int n_row_tiles, int n_col_tiles, EpiArgsT<OT> ep) {
   gemm_tc_body<T, OT, BN, EPI, 2>(map_a, map_b, K, n_row_tiles, n_col_tiles, ep);

@@ -70,7 +70,6 @@ k_gemm_bwd64(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
              int n_row_tiles, int n_col_tiles, Gemm64Args ep) {
   static_assert(sizeof(T) == 2, "16-bit activations only");
   static_assert(EPI == EPI_BWD_STATS || EPI == EPI_BWD_APPLY, "backward small-K epilogues only");
-  pdl_trigger();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   constexpr int BN = AW_G64_BN, BK = 64, NST = AW_G64_NST, NACT = gemm64_nact(EPI);
@@ -112,7 +111,6 @@ k_gemm_bwd64(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
 
   if (warp == 0) {
     // ------------------- TMA producer: operands and the activation tile of every tile -------------------

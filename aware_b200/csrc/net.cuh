@@ -69,7 +69,6 @@ __global__ void __launch_bounds__(128) k_mel(const float* __restrict__ mag, int 
                                              SparseMel sm, float* __restrict__ M,
                                              double* __restrict__ chan_part,
                                              const unsigned long long* __restrict__ peak_y) {
-  pdl_enter();
   extern __shared__ float s_a[];   // [AW_MEL_FRAMES][nb]
   const int clip = blockIdx.y, t0 = blockIdx.x * AW_MEL_FRAMES, c = threadIdx.x;
   const int nf = min(AW_MEL_FRAMES, T - t0);
@@ -154,7 +153,6 @@ __device__ __forceinline__ void sum_partials(const double* __restrict__ part, in
 // k_p0 then only streams.
 __global__ void __launch_bounds__(128) k_mel_stats(const double* __restrict__ chan_part, int nblk, int T,
                                                    ChanStats* __restrict__ cs, float* __restrict__ sigma_out) {
-  pdl_enter();
   __shared__ double s_red[32];
   const int clip = blockIdx.x, c = threadIdx.x;
   double s1, s2;
@@ -180,7 +178,6 @@ __global__ void __launch_bounds__(128) k_p0(const float* __restrict__ M, int T, 
                                             const ChanStats* __restrict__ cs,
                                             const float* __restrict__ sigma_in,
                                             AT* __restrict__ P0, int round_tf32) {
-  pdl_enter();
   const int clip = blockIdx.y, c = threadIdx.x, j0 = blockIdx.x * AW_P0_ROWS;
   const ChanStats st = cs[(long long)clip * AW_NMEL + c];
   const float fmu = st.mu, fr = st.rstd;
@@ -223,7 +220,6 @@ template <int MODE>
 __global__ void __launch_bounds__(256) k_finalize(const float* __restrict__ part, int ldp, int tiles,
                                                   int C, int Tp, float* __restrict__ stat,
                                                   double* __restrict__ raw = nullptr) {
-  pdl_enter();
   __shared__ double s_s[8][32][2];
   const int clip = blockIdx.y, cl = threadIdx.x & 31, sl = threadIdx.x >> 5;
   const int c = blockIdx.x * 32 + cl;
@@ -264,7 +260,6 @@ __global__ void __launch_bounds__(256) k_finalize(const float* __restrict__ part
 template <int MODE>
 __global__ void __launch_bounds__(256) k_finalize_small(const float* __restrict__ part, int ldp, int tiles,
                                                         int C, int Tp, float* __restrict__ stat) {
-  pdl_enter();
   const int clip = blockIdx.y, c = blockIdx.x * 256 + threadIdx.x;
   if (c >= C) return;
   const float* p0 = part + (((long long)clip * tiles) * ldp + c) * 2;
@@ -379,7 +374,6 @@ template <typename AT, int MODE>
 __global__ void __launch_bounds__(128) k_norm_rows(AT* __restrict__ X, const AT* __restrict__ P, int C,
                                                    int Tp, int Tp_pad, const float* __restrict__ stat,
                                                    const float* __restrict__ bstat, int round_tf32) {
-  pdl_enter();
   constexpr int V = Vec16<AT>::N;
   const int clip = blockIdx.z;
   // narrow layers (C / V < 128 column groups, e.g. the 64-channel last layer): the block's 128 threads are
@@ -464,7 +458,6 @@ struct HeadArgs {
 
 template <typename AT>
 __global__ void __launch_bounds__(256) k_head_partial(HeadArgs<AT> a) {
-  pdl_enter();
   __shared__ double s_acc[4][64][3];
   const int tile = blockIdx.x, clip = blockIdx.y, tid = threadIdx.x;
   const int c = tid & 63, g = tid >> 6;
@@ -494,7 +487,6 @@ __global__ void __launch_bounds__(256) k_head_partial(HeadArgs<AT> a) {
 
 template <typename AT>
 __global__ void __launch_bounds__(64) k_head_final(HeadArgs<AT> a, int tiles) {
-  pdl_enter();
   __shared__ float s_z[64], s_dz[64];
   const int clip = blockIdx.x, c = threadIdx.x;
   double sp = 0.0, sn = 0.0, np_ = 0.0;
@@ -566,7 +558,6 @@ __global__ void __launch_bounds__(64) k_head_final(HeadArgs<AT> a, int tiles) {
 
 template <typename AT>
 __global__ void __launch_bounds__(256) k_head_seed(HeadArgs<AT> a) {
-  pdl_enter();
   const int tile = blockIdx.x, clip = blockIdx.y, tid = threadIdx.x;
   const int c = tid & 63, g = tid >> 6;
   const float4 k = *reinterpret_cast<const float4*>(a.hcoef + ((long long)clip * 64 + c) * 4);
@@ -603,7 +594,6 @@ __global__ void __launch_bounds__(128) k_p0_bwd_reduce(const float* __restrict__
                                                        int Tp_pad, const ChanStats* __restrict__ cs,
                                                        double* __restrict__ bpart,
                                                        const float* __restrict__ gsc) {
-  pdl_enter();
   const int clip = blockIdx.y, c = threadIdx.x, t0 = blockIdx.x * AW_P0B_FRAMES;
   const float ginv = 1.0f / gsc[clip];                     // exact: the scale is a power of two
   const ChanStats st = cs[(long long)clip * AW_NMEL + c];
@@ -650,7 +640,6 @@ __global__ void __launch_bounds__(128) k_p0_bwd_coef(const double* __restrict__ 
                                                      const float* __restrict__ sigma_in,
                                                      P0BwdCoef* __restrict__ coef,
                                                      P0BwdScal* __restrict__ scal) {
-  pdl_enter();
   __shared__ double s_red[32];
   __shared__ float s_ab[3];
   const int clip = blockIdx.x, c = threadIdx.x;
@@ -689,7 +678,6 @@ __global__ void __launch_bounds__(128) k_p0_bwd_apply(const float* __restrict__ 
                                                       const float* __restrict__ mag_un,
                                                       double* __restrict__ s2_part,
                                                       const float* __restrict__ gsc) {
-  pdl_enter();
   __shared__ double s_red[32];
   __shared__ float s_dm[AW_P0A_FRAMES][AW_NMEL];
   const int clip = blockIdx.y, c = threadIdx.x, t0 = blockIdx.x * AW_P0A_FRAMES;

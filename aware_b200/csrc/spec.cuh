@@ -240,7 +240,6 @@ __global__ void __launch_bounds__(128) k_clip_scalars(const unsigned long long* 
                                                       int n_clips, ClipScal* __restrict__ out, int n_base = 0,
                                                       unsigned* __restrict__ dmax2 = nullptr,
                                                       const int* __restrict__ it_ptr = nullptr) {
-  pdl_enter();
   const int clip = blockIdx.x * blockDim.x + threadIdx.x;
   if (clip >= n_clips) return;
   // spectc.cuh: the slot that this iteration's k_tc_dsprep accumulates max |dA| into (next iteration's scale)
@@ -324,7 +323,6 @@ struct SpecArgs {
 
 template <int MODE, int K2LO, int K2HI>
 __global__ void __launch_bounds__(32 * AW_SP_WARPS, 2) k_spec(SpecArgs a) {
-  pdl_enter();
   extern __shared__ float smem[];
   float* s_buf = smem;                                   // [61 hops][256]
   float* s_win = s_buf + AW_SP_BUF;                      // [1024]

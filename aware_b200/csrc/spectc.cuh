@@ -153,7 +153,6 @@ __global__ void __launch_bounds__(256) k_tc_absmax(const float* __restrict__ dA,
 __global__ void __launch_bounds__(256) k_tc_dsprep(const float* __restrict__ dA, const float2* __restrict__ q, int T,
                                                    int nb, unsigned* __restrict__ dmax2, const int* __restrict__ it_ptr,
                                                    int n_clips, __half* __restrict__ dS) {
-  pdl_enter();
   __shared__ float s_mx[8];
   const int clip = blockIdx.y, t0 = blockIdx.x * AW_TC_FR;
   const int nf = min(AW_TC_FR, T - t0);
@@ -238,7 +237,6 @@ __device__ __forceinline__ void tc_nadam(float g, float& m1, float& v1, float& c
 // One thread = one bin of one frame; a block = AW_TC_FR consecutive frames of a clip (contiguous in the
 // [T][nb] state arrays).  All loads of an element are issued before its first store.
 __global__ void __launch_bounds__(256) k_tc_update(TcUpdateArgs a) {
-  pdl_enter();
   const int clip = blockIdx.y, t0 = blockIdx.x * AW_TC_FR, T = a.T, nb = a.nb;
   const int nf = min(AW_TC_FR, T - t0);
   const int it = *a.it_ptr;

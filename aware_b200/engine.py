@@ -115,13 +115,6 @@ class Engine:
         """16-bit loops: backward K = 64 layer on the TMA-streaming kernel (gemm64.cuh); off = generic GEMM epilogues."""
         _lib.check(self.lib.aw_ctx_set_option(self._ctx, _lib.OPT_BWD64_STREAM, 1.0 if on else 0.0))
 
-    def set_fuse_norm(self, forward: bool = True, backward: bool = True, pair: bool = False):
-        """16-bit loops: InstanceNorm (+ LeakyReLU) / its adjoint inside the K >= 512 GEMMs (accumulator held in
-        TMEM across the exchange of the clip's column sums); off (the default: measured a wash at 256 clips,
-        -5 % at <= 8 clips) = GEMM + finalize + stand-alone apply pass."""
-        v = (1 if forward else 0) | (2 if backward else 0) | (4 if pair else 0)
-        _lib.check(self.lib.aw_ctx_set_option(self._ctx, _lib.OPT_FUSE_NORM, float(v)))
-
     def detect_stats(self):
         """(clips seen by detect, clips re-evaluated exactly) since the engine was created."""
         out = []

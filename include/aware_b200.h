@@ -74,13 +74,9 @@ int64_t aw_launch_count(aw_ctx* ctx);
  * staging half of the weight tile) when the batch has an even number of 128-row tiles; results are
  * bit-identical to the one-CTA kernel.  AW_OPT_BWD64_STREAM (default 1): in the 16-bit loops the backward
  * K = 64 layer runs on k_gemm_bwd64 (csrc/gemm64.cuh: activation tiles streamed through a TMA ring, output
- * through a TMA bulk store) instead of the generic GEMM's statistics / apply epilogues.
- * AW_OPT_FUSE_NORM (default 0 -- measured a wash at 256 clips, see DESIGN.md): in the 16-bit loops the K >= 512 layers apply InstanceNorm + LeakyReLU
- * (bit 0, forward) and the InstanceNorm adjoint (bit 1, backward) inside the GEMM epilogue -- the accumulator
- * stays in TMEM while the CTAs holding the clip's other row tiles exchange their column sums -- so the raw
- * layer output is never written and the stand-alone finalize / apply passes disappear; bit 2: on CTA pairs. */
+ * through a TMA bulk store) instead of the generic GEMM's statistics / apply epilogues. */
 enum { AW_OPT_THRESHOLD = 0, AW_OPT_EXACT_MARGIN = 1, AW_OPT_TC_SPECTRAL = 2, AW_OPT_TWO_PASS = 3,
-       AW_OPT_PAIR_GEMM = 4, AW_OPT_BWD64_STREAM = 5, AW_OPT_FUSE_NORM = 6 };
+       AW_OPT_PAIR_GEMM = 4, AW_OPT_BWD64_STREAM = 5 };
 int aw_ctx_set_option(aw_ctx* ctx, int option, double value);
 /* counters since context creation: clips seen by aw_detect_batch / clips it re-evaluated exactly */
 enum { AW_STAT_DETECT_CLIPS = 0, AW_STAT_REEVAL_CLIPS = 1 };

@@ -157,87 +157,3 @@ def quick():
 
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "quick":
     quick()
-
-
-def fuse():
-    """fp16 loop at 256 clips x 10 s: InstanceNorm inside the K >= 512 GEMMs (EPI_*_FUSE) off / forward / both /
-    both on CTA pairs, alternating on the same box: graph-replay ms per iteration and instrumented classes"""
-    from aware_b200.synth import synth_batch, synth_bits
-    from aware_b200.utils.models import load
-    emb, det = load(); emb.verbose = False
-    eng = emb.engine
-    sr = 44100
-    n = int(os.environ.get("CLIPS", "256"))
-    x = torch.from_numpy(synth_batch(n, 10.0, sr)).cuda()
-    pat = torch.from_numpy(2 * synth_bits(n) - 1)
-    modes = [("off", dict(forward=False, backward=False)), ("fwd", dict(forward=True, backward=False)),
-             ("bwd", dict(forward=False, backward=True)),
-             ("both", dict(forward=True, backward=True)), ("pair", dict(forward=True, backward=True, pair=True))]
-    sel = os.environ.get("MODES")
-    if sel:
-        modes = [m for m in modes if m[0] in sel.split(",")]
-    for rep in range(2):
-        for name, kw in modes:
-            eng.set_fuse_norm(**kw)
-            eng.embed(x, sr, pat, iters=4, precision="fp16")
-            torch.cuda.synchronize()
-            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record()
-            eng.embed(x, sr, pat, iters=100, precision="fp16")
-            b.record()
-            torch.cuda.synchronize()
-            print("fuse=%-4s: %.3f ms per iteration (graph replay, 100 iterations)" % (name, a.elapsed_time(b) / 100), flush=True)
-    for name, kw in modes:
-        eng.set_fuse_norm(**kw)
-        eng.profile(True)
-        eng.embed(x, sr, pat, iters=10, precision="fp16")
-        torch.cuda.synchronize()
-        eng.profile(False)
-        eng.profile_read()
-        t = eng.profile_read_named()
-        tot = sum(v[1] for v in t.values())
-        print("fuse=%s instrumented total %.2f ms per iteration" % (name, tot / 10))
-        for k, v in sorted(t.items(), key=lambda kv: -kv[1][1])[:16]:
-            print("   %-28s %4d launches %8.3f ms/iter" % (k, v[0], v[1] / 10), flush=True)
-    eng.set_fuse_norm(False, False)
-
-
-if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "fuse":
-    fuse()
-
-
-def fusecheck():
-    """is the fused InstanceNorm forward as accurate as the separate passes?  per-clip losses of the first forward
-    pass and the first gradient, both against the exact fp32 path, at a clip count large enough to average the
-    LeakyReLU-kink noise"""
-    import numpy as np
-    from aware_b200.synth import synth_batch, synth_bits
-    from aware_b200.utils.models import load
-    emb, det = load(); emb.verbose = False
-    eng = emb.engine
-    sr = 44100
-    n = int(os.environ.get("CLIPS", "24"))
-    secs = float(os.environ.get("SECS", "3.1"))
-    x = torch.from_numpy(synth_batch(n, secs, sr)).cuda()
-    pat = torch.from_numpy(2 * synth_bits(n) - 1)
-    T = 1 + x.shape[1] // 256
-    def run(prec):
-        _, _, losses = eng.embed(x, sr, pat, iters=1, return_losses=True, precision=prec)
-        m = eng.embed_state("m", n, T, sr).cpu().numpy().astype(np.float64)
-        return losses[0].cpu().numpy().astype(np.float64), m
-    lx, mx = run("fp32")
-    for prec in ("fp16", "bf16"):
-        for name, kw in (("off", dict(forward=False, backward=False)), ("fwd", dict(forward=True, backward=False)),
-                         ("bwd", dict(forward=False, backward=True)), ("both", dict(forward=True, backward=True)),
-                         ("pair", dict(forward=True, backward=True, pair=True))):
-            eng.set_fuse_norm(**kw)
-            l, m = run(prec)
-            per = np.sqrt(((m - mx) ** 2).mean(axis=(1, 2)) / (mx ** 2).mean(axis=(1, 2)))
-            print("%s fuse=%-4s: loss err rms %.3e max %.3e | gradient rel RMS err: all %.4f, per clip median %.4f min %.4f max %.4f"
-                  % (prec, name, np.sqrt(((l - lx) ** 2).mean()), np.abs(l - lx).max(),
-                     np.sqrt(((m - mx) ** 2).mean() / (mx ** 2).mean()), np.median(per), per.min(), per.max()), flush=True)
-    eng.set_fuse_norm(False, False)
-
-
-if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "fusecheck":
-    fusecheck()

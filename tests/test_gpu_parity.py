@@ -1013,52 +1013,3 @@ def test_streaming_k64_backward_kernel_matches_the_generic_epilogues(eng, precis
         assert err.max() <= (2e-3 if precision == "fp16" else 2e-2)
         assert np.sqrt((err ** 2).mean()) <= (1e-4 if precision == "fp16" else 1e-3)
         assert np.abs(out[True][1] - out[False][1]).max() <= 5e-3
-
-
-@pytest.mark.parametrize("precision", ["fp16", "bf16"])
-def test_fused_instance_norm_gemm_matches_the_separate_passes(eng, precision):
-    """EPI_FWD_FUSE / EPI_BWD_FUSE (csrc/gemm.cuh): InstanceNorm + LeakyReLU and the InstanceNorm adjoint applied
-    inside the K >= 512 GEMMs -- the accumulator stays in TMEM while the CTAs that hold the clip's other row tiles
-    exchange their column sums -- against GEMM + finalize + stand-alone apply pass.  Same products and the same
-    float64 statistics; the fused form normalises the fp32 accumulator instead of the stored 16-bit H / dHhat, so
-    it can only be closer to the oracle.  16-bit rounding of H moves pre-activations across the LeakyReLU kink, so the
-    two forms are not compared with each other but both with the exact fp32 path from the same state: the first-moment
-    estimate after ONE step (m = 0.1 g) must be as close to it as the separate passes are; plus the losses of three
-    iterations, clip lengths with 2, 3 and 7 row tiles per clip (pad rows must
-    come out zero), odd and even clip counts, single CTAs and CTA pairs, forward only / backward only / both."""
-    sr = 44100
-    for secs, n_clips in ((1.5, 11), (3.1, 12), (10.0, 6)):
-        x = _clips(list(range(n_clips)), secs, sr)
-        xd = torch.from_numpy(x).cuda()
-        pat = torch.from_numpy(np.stack([O.encode_bits(b) for b in O.synth_bits(n_clips)]))
-        T = 1 + x.shape[1] // 256
-        out = {}
-        try:
-            for key, kw in (("off", dict(forward=False, backward=False)),
-                            ("fwd", dict(forward=True, backward=False)),
-                            ("bwd", dict(forward=False, backward=True)),
-                            ("both", dict(forward=True, backward=True)),
-                            ("pair", dict(forward=True, backward=True, pair=True))):
-                eng.set_fuse_norm(**kw)
-                eng.embed(xd, sr, pat, iters=1, precision=precision)
-                m = eng.embed_state("m", n_clips, T, sr).cpu().numpy()
-                _, _, losses = eng.embed(xd, sr, pat, iters=3, return_losses=True, precision=precision)
-                out[key] = (m, losses[:3].cpu().numpy())
-        finally:
-            eng.set_fuse_norm(False, False)
-        # yardstick: the exact fp32 path (float64-accumulated CUDA-core GEMMs) from the same state
-        eng.embed(xd, sr, pat, iters=1, precision="fp32")
-        mx = eng.embed_state("m", n_clips, T, sr).cpu().numpy()
-        rel = lambda a_: float(np.sqrt(((a_ - mx) ** 2).mean()) / np.sqrt((mx ** 2).mean()))
-        e_off = rel(out["off"][0])
-        for key in ("fwd", "bwd", "both", "pair"):
-            m1 = out[key][0]
-            assert np.isfinite(m1).all() and np.abs(m1).max() > 0
-            e1 = rel(m1)
-            print("fused IN %-4s (%s, %.1f s x %d): gradient rel. RMS error vs exact fp32 %.4f (separate passes %.4f), "
-                  "first loss %.6f / %.6f" % (key, precision, secs, n_clips, e1, e_off,
-                                                out[key][1][0].mean(), out["off"][1][0].mean()))
-            assert e1 <= 1.2 * e_off + 2e-3          # per-clip kink noise: +-20 % on a single short clip, +-1 % over 24
-            # first loss: same forward up to 16-bit rounding of H; iterations 2-3 already diverge through NAdam's sign step
-            assert np.abs(out[key][1][0] - out["off"][1][0]).max() <= (1e-4 if precision == "fp16" else 1e-3)
-            assert np.abs(out[key][1] - out["off"][1]).max() <= (1e-2 if precision == "fp16" else 3e-2)

@@ -34,7 +34,7 @@ def test_python_constants_equal_the_header_enums():
     from aware_b200 import _lib
     header = open(os.path.join(ROOT, "include", "aware_b200.h")).read()
     enums = {m.group(1): int(m.group(2)) for m in re.finditer(r"\bAW_((?:PREC|OPT|STAT|COMM)_[A-Z0-9_]+)\s*=\s*(\d+)", header)}
-    assert len(enums) >= 17 and "OPT_FUSE_NORM" in enums
+    assert len(enums) >= 16 and "OPT_BWD64_STREAM" in enums
     for name, value in enums.items():
         assert getattr(_lib, name) == value, name
     # multiply-shift division used by the frame-row kernels (csrc/spectc.cuh: e / nb == (e * magic) >> 32)
