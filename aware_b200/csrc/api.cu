@@ -116,7 +116,6 @@ struct aw_ctx {
   // clip; per-clip statistics are all-reduced over the ranks through the caller's callbacks
   struct Shard {
     aw_comm comm;
-    int T_glob, Tp_glob;       // frames / pooled frames of the whole clip
     int e0;                    // global index of the segment's first frame
     int own_lo, own_hi;        // frames this rank owns, LOCAL indices into the segment
     int64_t n_allreduce = 0, n_allgather = 0;
@@ -286,6 +285,23 @@ static int sh_halo_exchange(aw_ctx* ctx, float* arr, int nb, cudaStream_t st) {
   ctx->launches += 2;
   AW_LAUNCH_CHECK();
   prof_mark(ctx, st, nullptr);
+  return 0;
+}
+
+// ---- the places where the frame-sharded mode differs from a batch; no-ops for whole clips
+static int sync_peak(aw_ctx* ctx, unsigned long long* peak, cudaStream_t st) {
+  return ctx->sh ? sh_peak_max(ctx, peak, st) : 0;
+}
+static int sync_halo(aw_ctx* ctx, float* arr, int nb, cudaStream_t st) {
+  return ctx->sh ? sh_halo_exchange(ctx, arr, nb, st) : 0;
+}
+// [clip][nblk][W] partial sums -> what a per-clip consumer reads: grouped when long (whole clips), or
+// summed over the whole clip into one block (frame-sharded mode)
+static int clip_sums(aw_ctx* ctx, Buf& scratch, const double*& part, int& nblk, int n_clips, int W, cudaStream_t st) {
+  if (!ctx->sh) return reduce_if_long(ctx, scratch, part, nblk, n_clips, W, st);
+  if (sh_reduce_sum(ctx, scratch, part, nblk, W, st)) return 1;
+  part = sh_red(ctx);
+  nblk = 1;
   return 0;
 }
 
@@ -764,18 +780,25 @@ static int get_mel(aw_ctx* ctx, int bin0, int nbins, SparseMel* out) {
 // ---------------------------------------------------------------------------
 struct Dims {
   int n, N, T, L, Tp, Tp_pad, tiles, rows, bin0, nb;
+  int T_clip, Tp_clip;   // frames / pooled frames per-clip statistics divide by: the whole clip's, also for a shard
 };
+
+static void set_frames(Dims* d, int T) {
+  d->T = T;
+  d->L = AW_HOP * (T - 1);
+  d->Tp = T / 2;
+  d->Tp_pad = (d->Tp + AW_ROW_TILE - 1) / AW_ROW_TILE * AW_ROW_TILE;
+  d->tiles = d->Tp_pad / AW_ROW_TILE;
+  d->rows = d->n * d->Tp_pad;
+  d->T_clip = T;
+  d->Tp_clip = d->Tp;
+}
 
 static int make_dims(aw_ctx* ctx, int n, int N, int sr, Dims* d) {
   AW_REQUIRE(n >= 1, "n_clips must be >= 1");
   AW_REQUIRE(N > 1024, "clips must be longer than 1024 samples (got %d)", N);
   d->n = n; d->N = N;
-  d->T = 1 + N / AW_HOP;
-  d->L = AW_HOP * (d->T - 1);
-  d->Tp = d->T / 2;
-  d->Tp_pad = (d->Tp + AW_ROW_TILE - 1) / AW_ROW_TILE * AW_ROW_TILE;
-  d->tiles = d->Tp_pad / AW_ROW_TILE;
-  d->rows = n * d->Tp_pad;
+  set_frames(d, 1 + N / AW_HOP);
   return aw_band_bins(ctx, sr, &d->bin0, &d->nb);
 }
 
@@ -818,11 +841,13 @@ static Acc acc_view(aw_ctx* ctx, const Dims& d) {
   return a;
 }
 
-static int ensure_net_ws(aw_ctx* ctx, const Dims& d, bool backward) {
+// ds: the frames the spectra span, d: the frames the detector net runs on (the same dims for whole
+// clips; a shard's segment and its own frames)
+static int ensure_net_ws(aw_ctx* ctx, const Dims& ds, const Dims& d, bool backward) {
   const size_t n = d.n, R = d.rows;
-  if (ensure(ctx->accum, acc_doubles(d) * 8)) return 1;
+  if (ensure(ctx->accum, acc_doubles(ds) * 8)) return 1;
   if (ensure(ctx->peakx, n * 8)) return 1;
-  if (ensure(ctx->mag, n * d.T * d.nb * 4)) return 1;
+  if (ensure(ctx->mag, n * ds.T * ds.nb * 4)) return 1;
   if (ensure(ctx->M, n * d.T * AW_NMEL * 4)) return 1;
   if (ensure(ctx->cs, n * AW_NMEL * sizeof(ChanStats))) return 1;
   if (ensure(ctx->sigma, n * 4)) return 1;
@@ -957,13 +982,13 @@ static float* own_frames(aw_ctx* ctx, float* base, int nb) {
 }
 // frame-sharded InstanceNorm statistics: local raw sums -> all-reduce -> (mean, rstd) / adjoint means
 template <bool BWD>
-static int sh_finalize(aw_ctx* ctx, int C, int tiles, float* stat, cudaStream_t st) {
+static int sh_finalize(aw_ctx* ctx, const Dims& d, int C, float* stat, cudaStream_t st) {
   double* red = (double*)((uint8_t*)ctx->sh->comm.d_arena + AW_ARENA_RED);
-  k_finalize<2><<<dim3((C + 31) / 32, 1), 256, 0, st>>>((float*)ctx->part.p, C, tiles, C, 1, nullptr, red);
+  k_finalize<2><<<dim3((C + 31) / 32, 1), 256, 0, st>>>((float*)ctx->part.p, C, d.tiles, C, 1, nullptr, red);
   ctx->launches++;
   AW_LAUNCH_CHECK();
   if (sh_allreduce(ctx, 2 * (int64_t)C, AW_COMM_F64, AW_COMM_SUM, st)) return 1;
-  k_stat_from_sums<BWD><<<dim3((C + 255) / 256, 1), 256, 0, st>>>(red, C, ctx->sh->Tp_glob, stat);
+  k_stat_from_sums<BWD><<<dim3((C + 255) / 256, 1), 256, 0, st>>>(red, C, d.Tp_clip, stat);
   ctx->launches++;
   AW_LAUNCH_CHECK();
   return 0;
@@ -984,13 +1009,9 @@ static int net_forward(aw_ctx* ctx, const Dims& d, const Acc& acc, const SparseM
     dim3 g2((d.Tp_pad + AW_P0_ROWS - 1) / AW_P0_ROWS, d.n);
     const double* cp = acc.chan_part;
     int cb = acc.mel_blocks;
-    if (ctx->sh) {            // channel sums over the WHOLE clip
-      if (sh_reduce_sum(ctx, ctx->red_a, cp, cb, 2 * AW_NMEL, st)) return 1;
-      cp = sh_red(ctx);
-      cb = 1;
-    } else if (reduce_if_long(ctx, ctx->red_a, cp, cb, d.n, 2 * AW_NMEL, st)) return 1;
+    if (clip_sums(ctx, ctx->red_a, cp, cb, d.n, 2 * AW_NMEL, st)) return 1;   // channel sums over the WHOLE clip
     prof_mark(ctx, st, "mel_stats");
-    k_mel_stats<<<d.n, 128, 0, st>>>(cp, cb, ctx->sh ? ctx->sh->T_glob : d.T, (ChanStats*)ctx->cs.p, (float*)ctx->sigma.p);
+    k_mel_stats<<<d.n, 128, 0, st>>>(cp, cb, d.T_clip, (ChanStats*)ctx->cs.p, (float*)ctx->sigma.p);
     ctx->launches++;
     AW_LAUNCH_CHECK();
     prof_mark(ctx, st, "p0");
@@ -1020,7 +1041,7 @@ static int net_forward(aw_ctx* ctx, const Dims& d, const Acc& acc, const SparseM
     dim3 g((cout + 31) / 32, d.n);
     prof_mark(ctx, st, "finalize_fwd");
     if (ctx->sh) {
-      if (sh_finalize<false>(ctx, cout, d.tiles, (float*)ctx->stat[l + 1].p, st)) return 1;
+      if (sh_finalize<false>(ctx, d, cout, (float*)ctx->stat[l + 1].p, st)) return 1;
     } else {
       if (d.tiles <= 16)
         k_finalize_small<0><<<dim3((cout + 255) / 256, d.n), 256, 0, st>>>((float*)ctx->part.p, cout, d.tiles, cout,
@@ -1091,7 +1112,7 @@ static int net_backward(aw_ctx* ctx, const Dims& d, const Acc& acc, const Sparse
     dim3 g((n + 31) / 32, d.n);
     prof_mark(ctx, st, "finalize_bwd");
     if (ctx->sh) {
-      if (sh_finalize<true>(ctx, n, d.tiles, (float*)ctx->bstat.p, st)) return 1;
+      if (sh_finalize<true>(ctx, d, n, (float*)ctx->bstat.p, st)) return 1;
     } else {
       if (d.tiles <= 16)
         k_finalize_small<1><<<dim3((n + 255) / 256, d.n), 256, 0, st>>>((float*)ctx->part.p, n, d.tiles, n, d.Tp,
@@ -1151,13 +1172,9 @@ static int net_backward(aw_ctx* ctx, const Dims& d, const Acc& acc, const Sparse
   dim3 g2((d.T + AW_P0A_FRAMES - 1) / AW_P0A_FRAMES, d.n);
   const double* bp = acc.bpart;
   int bb = acc.p0b_blocks;
-  if (ctx->sh) {
-    if (sh_reduce_sum(ctx, ctx->red_b, bp, bb, 2 * AW_NMEL, st)) return 1;
-    bp = sh_red(ctx);
-    bb = 1;
-  } else if (reduce_if_long(ctx, ctx->red_b, bp, bb, d.n, 2 * AW_NMEL, st)) return 1;
+  if (clip_sums(ctx, ctx->red_b, bp, bb, d.n, 2 * AW_NMEL, st)) return 1;
   prof_mark(ctx, st, "p0_bwd_coef");
-  k_p0_bwd_coef<<<d.n, 128, 0, st>>>(bp, bb, ctx->sh ? ctx->sh->T_glob : d.T, (ChanStats*)ctx->cs.p, (float*)ctx->sigma.p,
+  k_p0_bwd_coef<<<d.n, 128, 0, st>>>(bp, bb, d.T_clip, (ChanStats*)ctx->cs.p, (float*)ctx->sigma.p,
                                      (P0BwdCoef*)ctx->p0coef.p, (P0BwdScal*)ctx->p0scal.p);
   ctx->launches++;
   AW_LAUNCH_CHECK();
@@ -1177,7 +1194,7 @@ static int run_head(aw_ctx* ctx, const Dims& d, const float* pattern, float* val
                     int n_total, bool backward, cudaStream_t st) {
   HeadArgs<AT> h;
   h.P4 = (AT*)ctx->act[4].p; h.Tp = d.Tp; h.Tp_pad = d.Tp_pad;
-  h.Tp_glob = ctx->sh ? ctx->sh->Tp_glob : d.Tp;
+  h.Tp_glob = d.Tp_clip;
   h.stat4 = (float*)ctx->stat[4].p;
   h.pattern = pattern; h.values = values; h.losses = losses;
   h.best = (float*)ctx->best.p; h.improved = (int*)ctx->improved.p;
@@ -1190,14 +1207,13 @@ static int run_head(aw_ctx* ctx, const Dims& d, const float* pattern, float* val
   h.hcoef = (float*)ctx->hcoef.p;
   prof_mark(ctx, st, "head");
   k_head_partial<AT><<<dim3(d.tiles, d.n), 256, 0, st>>>(h);
-  if (ctx->sh) {
-    if (sh_reduce_sum(ctx, ctx->red_a, h.hpart, d.tiles, 64 * 3, st)) return 1;
-    HeadArgs<AT> hf = h;
-    hf.hpart = const_cast<double*>(sh_red(ctx));
-    k_head_final<AT><<<d.n, 64, 0, st>>>(hf, 1);
-  } else {
-    k_head_final<AT><<<d.n, 64, 0, st>>>(h, d.tiles);
-  }
+  const double* hp = h.hpart;
+  int hb = d.tiles;
+  // k_head_final takes any number of tile partials: whole clips pass them on ungrouped
+  if (ctx->sh && clip_sums(ctx, ctx->red_a, hp, hb, d.n, 64 * 3, st)) return 1;
+  HeadArgs<AT> hf = h;
+  hf.hpart = const_cast<double*>(hp);
+  k_head_final<AT><<<d.n, 64, 0, st>>>(hf, hb);
   ctx->launches += 2;
   if (backward && pattern) {
     k_head_seed<AT><<<dim3(d.tiles, d.n), 256, 0, st>>>(h);
@@ -1306,32 +1322,36 @@ static int begin_pass(aw_ctx* ctx, int n, int* it, cudaStream_t st, unsigned* dm
   return 0;
 }
 
+// f(AT()) with the activation storage type of the context's precision
+template <typename F>
+static int with_act_type(aw_ctx* ctx, F&& f) {
+  if (ctx->prec == AW_PREC_BF16) return f(__nv_bfloat16());
+  if (ctx->prec == AW_PREC_FP16) return f(__half());
+  return f(float());
+}
+
 // ---------------------------------------------------------------------------
-static int detect_pipeline(aw_ctx* ctx, const float* d_audio, int n_clips, int n_samples, int64_t stride,
-                           int sample_rate, float* d_values, cudaStream_t st) {
-  Dims d;
-  if (make_dims(ctx, n_clips, n_samples, sample_rate, &d)) return 1;
-  if (ensure_net_ws(ctx, d, false)) return 1;
+// One detector pass over ds.n clips x (or over one shard's segment; see ensure_net_ws for ds / dn).
+static int detect_pass(aw_ctx* ctx, const Dims& ds, const Dims& dn, const float* x, int64_t stride, float* d_values,
+                       cudaStream_t st) {
+  if (ensure_net_ws(ctx, ds, dn, false)) return 1;
   SparseMel sm;
-  if (get_mel(ctx, d.bin0, d.nb, &sm)) return 1;
-  const Acc acc = acc_view(ctx, d);
-  if (begin_pass(ctx, d.n, nullptr, st)) return 1;
-  if (launch_peak(ctx, d_audio, stride, n_samples, d.n, (unsigned long long*)ctx->peakx.p, st)) return 1;
-  AnaArgs a = ana_base(ctx, d);
-  a.sig = d_audio; a.sig_stride = stride; a.len = n_samples;
-  a.peak = (unsigned long long*)ctx->peakx.p;
+  if (get_mel(ctx, ds.bin0, ds.nb, &sm)) return 1;
+  const Acc acc = acc_view(ctx, dn);
+  unsigned long long* peak = (unsigned long long*)ctx->peakx.p;
+  if (begin_pass(ctx, ds.n, nullptr, st)) return 1;
+  if (launch_peak(ctx, x, stride, ds.N, ds.n, peak, st)) return 1;
+  if (sync_peak(ctx, peak, st)) return 1;        // waveform.py:19 over the whole clip
+  AnaArgs a = ana_base(ctx, ds);
+  a.sig = x; a.sig_stride = stride; a.len = ds.N;
+  a.peak = peak;
   a.mag = (float*)ctx->mag.p;
-  if (launch_ana<ANA_MAG>(ctx, d, a, st)) return 1;
-  if (ctx->prec == AW_PREC_BF16) {
-    if (net_forward<__nv_bfloat16>(ctx, d, acc, sm, st)) return 1;
-    return run_head<__nv_bfloat16>(ctx, d, nullptr, d_values, nullptr, d.n, false, st);
-  }
-  if (ctx->prec == AW_PREC_FP16) {
-    if (net_forward<__half>(ctx, d, acc, sm, st)) return 1;
-    return run_head<__half>(ctx, d, nullptr, d_values, nullptr, d.n, false, st);
-  }
-  if (net_forward<float>(ctx, d, acc, sm, st)) return 1;
-  return run_head<float>(ctx, d, nullptr, d_values, nullptr, d.n, false, st);
+  if (launch_ana<ANA_MAG>(ctx, ds, a, st)) return 1;
+  return with_act_type(ctx, [&](auto tag) -> int {
+    using AT = decltype(tag);
+    if (net_forward<AT>(ctx, dn, acc, sm, st)) return 1;
+    return run_head<AT>(ctx, dn, nullptr, d_values, nullptr, dn.n, false, st);
+  });
 }
 
 // flags[0] = number of clips with min_i |v_i - thr| < margin, flags[1 + clip] = 1 for those clips
@@ -1361,7 +1381,9 @@ extern "C" int aw_detect_batch(aw_ctx* ctx, const float* d_audio, int n_clips, i
   AW_ENTRY("aw_detect_batch");
   nvtxRangePushA("aw_detect_batch");
   struct Pop { ~Pop() { nvtxRangePop(); } } pop_;
-  if (detect_pipeline(ctx, d_audio, n_clips, n_samples, stride, sample_rate, d_values, st)) return 1;
+  Dims d;
+  if (make_dims(ctx, n_clips, n_samples, sample_rate, &d)) return 1;
+  if (detect_pass(ctx, d, d, d_audio, stride, d_values, st)) return 1;
   ctx->stat_detect_clips += n_clips;
   if (ctx->prec == AW_PREC_FP32 || ctx->exact_margin <= 0.0) {
     prof_mark(ctx, st, nullptr);
@@ -1390,11 +1412,13 @@ extern "C" int aw_detect_batch(aw_ctx* ctx, const float* d_audio, int n_clips, i
   nvtxRangePushA("exact_reevaluation");
   const int prev = ctx->prec;
   ctx->prec = AW_PREC_FP32;
+  Dims d1 = d;
+  d1.n = 1;
+  d1.rows = d1.Tp_pad;
   int rc = 0;
   for (int i = 0; i < n_clips && !rc; ++i)
     if (ctx->h_lowm[1 + i])
-      rc = detect_pipeline(ctx, d_audio + (size_t)i * stride, 1, n_samples, stride, sample_rate,
-                           d_values + (size_t)i * AW_NBITS, st);
+      rc = detect_pass(ctx, d1, d1, d_audio + (size_t)i * stride, stride, d_values + (size_t)i * AW_NBITS, st);
   ctx->prec = prev;
   nvtxRangePop();
   prof_mark(ctx, st, nullptr);
@@ -1577,6 +1601,196 @@ static int tc_backward(aw_ctx* ctx, const Dims& d, int* itc, cudaStream_t st, in
   return 0;
 }
 
+// Workspace of an embed call (see ensure_net_ws for ds / dn), the NAdam step table and n_flags cleared
+// non-finite flags.
+static int embed_setup(aw_ctx* ctx, const Dims& ds, const Dims& dn, int n_flags, int iters, cudaStream_t st) {
+  if (ensure_net_ws(ctx, ds, dn, true)) return 1;
+  const size_t sp = (size_t)ds.n * ds.T * ds.nb;
+  if (ensure(ctx->ph_u, sp * 8) || ensure(ctx->ph_q, sp * 8) || ensure(ctx->c0, sp * 4) ||
+      ensure(ctx->c, sp * 4) || ensure(ctx->m, sp * 4) || ensure(ctx->v, sp * 4) ||
+      ensure(ctx->cbest, sp * 4) || ensure(ctx->dA, sp * 4) ||
+      ensure(ctx->yoob, (size_t)ds.n * ds.L * 4) || ensure(ctx->y, (size_t)ds.n * ds.L * 4) ||
+      ensure(ctx->zoob, (size_t)ds.n * ds.L * 4) ||
+      ensure(ctx->pattern, (size_t)ds.n * AW_NBITS * 4) || ensure(ctx->scal, (size_t)ds.n * sizeof(ClipScal)) ||
+      ensure(ctx->nonfinite, (size_t)n_flags * 4) || ensure(ctx->smax, (size_t)ds.n * 4) ||
+      ensure(ctx->steps, (size_t)(iters > 0 ? iters : 1) * sizeof(NadamStep)))
+    return 1;
+  std::vector<NadamStep> tab;
+  nadam_table(iters, tab);
+  if (iters > 0)
+    AW_CUDA(cudaMemcpyAsync(ctx->steps.p, tab.data(), tab.size() * sizeof(NadamStep),
+                            cudaMemcpyHostToDevice, st));
+  AW_CUDA(cudaMemsetAsync(ctx->nonfinite.p, 0, (size_t)n_flags * 4, st));
+  ctx->last_embed_clips = n_flags;
+  AW_CUDA(cudaStreamSynchronize(st));   // `tab` is pageable host memory
+  return 0;
+}
+
+// What one embed wave reads and writes, offset to the wave's first clip.
+struct WaveIO {
+  const float* x; int64_t stride;
+  const int32_t* pattern;                 // [n][AW_NBITS]
+  const float* scale; bool signed_max;    // output scale: per clip, the input's signed max (AW_SCALE_SIGNED_MAX) or none
+  float* out; int64_t out_stride;
+  // samples [pk_lo, pk_hi) compete for the peak and are written out (pk_hi = 0: all); the peak word packs
+  // local index + idx_base (frame-sharded mode: a segment's own samples, global indices)
+  int pk_lo, pk_hi, idx_base;
+  float* best_loss;                       // [n] or null
+  float* losses; int n_total;             // [iters][n_total] or null
+  int* nonfinite;                         // [n]
+};
+
+// One embed wave: init, the optimisation loop and the final synthesis of ds.n clips, or of one shard's
+// segment (see ensure_net_ws for ds / dn).
+static int embed_wave(aw_ctx* ctx, const Dims& ds, const Dims& dn, const WaveIO& w, int iters, bool use_graph,
+                      cudaStream_t st) {
+  SparseMel sm;
+  if (get_mel(ctx, ds.bin0, ds.nb, &sm)) return 1;
+  const Acc acc = acc_view(ctx, dn);           // peak word at the base; partial-sum arrays of the net's frames
+  unsigned long long* peakx = (unsigned long long*)ctx->peakx.p;
+  int* itc = (int*)ctx->itc.p;
+
+  k_set_int<<<1, 1, 0, st>>>(itc, -1);
+  k_fill<<<(ds.n + 255) / 256, 256, 0, st>>>((float*)ctx->best.p, INFINITY, ds.n);
+  k_pattern_to_float<<<(ds.n * AW_NBITS + 255) / 256, 256, 0, st>>>(w.pattern, (float*)ctx->pattern.p,
+                                                                      ds.n * AW_NBITS);
+  ctx->launches += 3;
+  AW_LAUNCH_CHECK();
+  if (launch_peak(ctx, w.x, w.stride, ds.N, ds.n, peakx, st, w.signed_max ? (int*)ctx->smax.p : nullptr)) return 1;
+  if (sync_peak(ctx, peakx, st)) return 1;
+
+  // ---- pre-STFT, bounds, constant out-of-band waveform (multibit_embedder.py:143-160)
+  nvtxRangePushA("embed:init_stft_bounds_oob");
+  AnaArgs a0 = ana_base(ctx, ds);
+  a0.sig = w.x; a0.sig_stride = w.stride; a0.len = ds.N;
+  a0.peak = peakx;
+  a0.mag = (float*)ctx->c0.p; a0.ph = (float2*)ctx->ph_u.p;
+  a0.c = (float*)ctx->c.p; a0.m = (float*)ctx->m.p; a0.v = (float*)ctx->v.p;
+  a0.cbest = (float*)ctx->cbest.p;
+  if (launch_ana<ANA_INIT>(ctx, ds, a0, st)) return 1;
+  SynArgs s0 = syn_base(ctx, ds);
+  s0.amp = (float*)ctx->c0.p; s0.ph = (float2*)ctx->ph_u.p; s0.scale = 1.0f / AW_NFFT;
+  s0.x = w.x; s0.x_stride = w.stride; s0.peak_x = peakx;
+  s0.y_oob = (float*)ctx->yoob.p;
+  s0.z_oob = (float*)ctx->zoob.p;
+  if (launch_syn<SYN_OOB>(ctx, ds, s0, st)) return 1;
+  // fp16 loop at 44.1 / 48 kHz: the loop's band-limited transforms run on the tensor cores (spectc.cuh)
+  const bool tc = tc_eligible(ctx, ds);
+  if (tc) {
+    if (tc_prepare_mats(ctx, ds, ctx->h_window.data())) return 1;
+    if (tc_setup_wave(ctx, ds, st)) return 1;
+  }
+  ctx->tc_active = tc;
+  struct TcOff { aw_ctx* c; ~TcOff() { c->tc_active = false; } } tc_off_{ctx};
+  nvtxRangePop();
+
+  // ---- optimisation loop (multibit_embedder.py:95-122)
+  nvtxRangePushA("embed:nadam_loop");
+  auto iteration = [&](bool first) -> int {
+    // fused spectral passes (spec.cuh): y and dpad never leave shared memory
+    if (begin_pass(ctx, ds.n, itc, st)) return 1;
+    if (tc) {
+      if (tc_forward(ctx, ds, acc, st)) return 1;
+    } else {
+      SpecArgs f;
+      memset(&f, 0, sizeof(f));
+      f.amp = (float*)ctx->c.p; f.ph = (float2*)ctx->ph_u.p;
+      f.z_oob = (float*)ctx->zoob.p; f.peak_y = acc.peak_y;
+      f.mag = (float*)ctx->mag.p; f.q = (float2*)ctx->ph_q.p;
+      f.pk_lo = w.pk_lo; f.pk_hi = w.pk_hi; f.idx_base = w.idx_base;
+      if (launch_spec<SPEC_FWD>(ctx, ds, f, st)) return 1;
+    }
+    if (sync_peak(ctx, acc.peak_y, st)) return 1;                      // max |y| over the whole clip
+    if (with_act_type(ctx, [&](auto tag) -> int {
+          using AT = decltype(tag);
+          if (net_forward<AT>(ctx, dn, acc, sm, st, acc.peak_y)) return 1;
+          if (run_head<AT>(ctx, dn, (float*)ctx->pattern.p, (float*)ctx->values.p, w.losses, w.n_total, true, st))
+            return 1;
+          return net_backward<AT>(ctx, dn, acc, sm, st, true);
+        }))
+      return 1;
+    const double* sp2 = acc.s2_part;
+    int sb2 = p0a_blocks(dn);
+    if (clip_sums(ctx, ctx->red_c, sp2, sb2, dn.n, 1, st)) return 1;                       // Euler sum over the clip
+    if (sb2 > 512 && reduce_if_long(ctx, ctx->red_a, sp2, sb2, dn.n, 1, st)) return 1;   // 1 h: 38 760 -> 606 -> 10
+    prof_mark(ctx, st, "clip_scalars");
+    k_clip_scalars<<<(dn.n + 127) / 128, 128, 0, st>>>(acc.peak_y, sp2, sb2, dn.n, (ClipScal*)ctx->scal.p, w.idx_base,
+                                                       tc ? (unsigned*)ctx->tc_dmax.p : nullptr, itc);
+    ctx->launches++;
+    AW_LAUNCH_CHECK();
+    if (sync_halo(ctx, (float*)ctx->dA.p, ds.nb, st)) return 1;       // spectral gradient of the halo frames
+    if (tc) return tc_backward(ctx, ds, itc, st, w.nonfinite, first);
+    SpecArgs b;
+    memset(&b, 0, sizeof(b));
+    b.amp = (float*)ctx->dA.p; b.ph = (float2*)ctx->ph_q.p;
+    b.scal = (ClipScal*)ctx->scal.p; b.u = (float2*)ctx->ph_u.p;
+    b.c = (float*)ctx->c.p; b.m = (float*)ctx->m.p; b.v = (float*)ctx->v.p;
+    b.cbest = (float*)ctx->cbest.p; b.c0 = (float*)ctx->c0.p;
+    b.improved = (int*)ctx->improved.p; b.steps = (NadamStep*)ctx->steps.p; b.it_ptr = itc;
+    b.nonfinite = w.nonfinite;
+    b.tol_ratio = (float)pow(10.0, -(double)ctx->tol_db / 20.0);
+    if (launch_spec<SPEC_BWD>(ctx, ds, b, st)) return 1;
+    return sync_halo(ctx, (float*)ctx->c.p, ds.nb, st);              // updated coefficients of the halo frames
+  };
+  if (use_graph) {
+    // iteration 0 runs eagerly (function attributes, scratch sizes), iteration 1 is captured
+    // without executing, and the graph is replayed for iterations 1 .. iters-1; the iteration
+    // index and all per-clip state live on the device, so every replay is identical work
+    const int64_t l0 = ctx->launches;
+    if (iteration(true)) return 1;
+    const int64_t per_iter = ctx->launches - l0 - (tc ? 1 : 0);
+    AW_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed));
+    const int rc = iteration(false);
+    cudaGraph_t graph = nullptr;
+    const cudaError_t ce = cudaStreamEndCapture(st, &graph);
+    if (rc || ce != cudaSuccess || !graph) {
+      if (graph) cudaGraphDestroy(graph);
+      return rc ? 1 : set_error("aw_embed_batch: stream capture failed: %s", cudaGetErrorString(ce));
+    }
+    cudaGraphExec_t exec = nullptr;
+    if (cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) {
+      cudaGraphDestroy(graph);
+      return set_error("aw_embed_batch: cudaGraphInstantiate failed: %s", cudaGetErrorString(cudaGetLastError()));
+    }
+    for (int it = 1; it < iters; ++it) {
+      if (cudaGraphLaunch(exec, st) != cudaSuccess) {
+        cudaGraphExecDestroy(exec);
+        cudaGraphDestroy(graph);
+        return set_error("aw_embed_batch: cudaGraphLaunch failed: %s", cudaGetErrorString(cudaGetLastError()));
+      }
+    }
+    ctx->launches += per_iter * (iters - 2);      // the captured pass was counted once already
+    cudaGraphExecDestroy(exec);
+    cudaGraphDestroy(graph);
+  } else {
+    for (int it = 0; it < iters; ++it)
+      if (iteration(it == 0)) return 1;
+  }
+  nvtxRangePop();
+  // ---- final synthesis from the best coefficients (multibit_embedder.py:173-192), peak over the whole clip
+  nvtxRangePushA("embed:final_synthesis");
+  if (sync_halo(ctx, (float*)ctx->cbest.p, ds.nb, st)) return 1;
+  if (begin_pass(ctx, ds.n, nullptr, st)) return 1;
+  SynArgs sf = syn_base(ctx, ds);
+  sf.amp = (float*)ctx->cbest.p; sf.ph = (float2*)ctx->ph_u.p; sf.scale = 1.0f / AW_NFFT;
+  sf.y_oob = (float*)ctx->yoob.p; sf.y = (float*)ctx->y.p; sf.peak_y = acc.peak_y;
+  sf.pk_lo = w.pk_lo; sf.pk_hi = w.pk_hi;
+  if (launch_syn<SYN_WAVE>(ctx, ds, sf, st)) return 1;
+  if (sync_peak(ctx, acc.peak_y, st)) return 1;
+  const int len = (w.pk_hi > 0 ? w.pk_hi : ds.L) - w.pk_lo;
+  dim3 g(std::min((len + 4095) / 4096, std::max(64, 8192 / ds.n)), ds.n);
+  prof_mark(ctx, st, "final_normalize");
+  k_final_normalize<<<g, 256, 0, st>>>((float*)ctx->y.p + w.pk_lo, len, acc.peak_y, w.scale,
+                                       w.signed_max ? (const int*)ctx->smax.p : nullptr, w.out, w.out_stride);
+  ctx->launches++;
+  AW_LAUNCH_CHECK();
+  if (w.best_loss)
+    AW_CUDA(cudaMemcpyAsync(w.best_loss, ctx->best.p, (size_t)ds.n * 4, cudaMemcpyDeviceToDevice, st));
+  ctx->last_n = ds.n; ctx->last_T = ds.T; ctx->last_nb = ds.nb;
+  nvtxRangePop();
+  return 0;
+}
+
 extern "C" int aw_embed_batch(aw_ctx* ctx, const float* d_audio, int n_clips, int n_samples,
                               int64_t stride, int sample_rate, const int32_t* d_pattern, int iters,
                               const float* d_scale, int scale_mode, float* d_out, int64_t out_stride,
@@ -1621,181 +1835,22 @@ extern "C" int aw_embed_batch(aw_ctx* ctx, const float* d_audio, int n_clips, in
   Dims d;
   if (make_dims(ctx, wave_clips, n_samples, sample_rate, &d)) return 1;
   AW_REQUIRE(out_stride >= d.L, "aw_embed_batch: out_stride %lld < %d", (long long)out_stride, d.L);
-  if (ensure_net_ws(ctx, d, true)) return 1;
-  const size_t sp = (size_t)d.n * d.T * d.nb;
-  if (ensure(ctx->ph_u, sp * 8) || ensure(ctx->ph_q, sp * 8) || ensure(ctx->c0, sp * 4) ||
-      ensure(ctx->c, sp * 4) || ensure(ctx->m, sp * 4) || ensure(ctx->v, sp * 4) ||
-      ensure(ctx->cbest, sp * 4) || ensure(ctx->dA, sp * 4) ||
-      ensure(ctx->yoob, (size_t)d.n * d.L * 4) || ensure(ctx->y, (size_t)d.n * d.L * 4) ||
-      ensure(ctx->zoob, (size_t)d.n * d.L * 4) ||
-      ensure(ctx->pattern, (size_t)d.n * AW_NBITS * 4) || ensure(ctx->scal, (size_t)d.n * sizeof(ClipScal)) ||
-      ensure(ctx->nonfinite, (size_t)n_clips * 4) || ensure(ctx->smax, (size_t)d.n * 4) ||
-      ensure(ctx->steps, (size_t)(iters > 0 ? iters : 1) * sizeof(NadamStep)))
-    return 1;
-  SparseMel sm;
-  if (get_mel(ctx, d.bin0, d.nb, &sm)) return 1;
-  std::vector<NadamStep> tab;
-  nadam_table(iters, tab);
-  if (iters > 0)
-    AW_CUDA(cudaMemcpyAsync(ctx->steps.p, tab.data(), tab.size() * sizeof(NadamStep),
-                            cudaMemcpyHostToDevice, st));
-  AW_CUDA(cudaMemsetAsync(ctx->nonfinite.p, 0, (size_t)n_clips * 4, st));
-  ctx->last_embed_clips = n_clips;
-  AW_CUDA(cudaStreamSynchronize(st));   // `tab` is pageable host memory
+  if (embed_setup(ctx, d, d, n_clips, iters, st)) return 1;
 
   for (int w0 = 0; w0 < n_clips; w0 += wave_clips) {
     Dims dw = d;
     dw.n = std::min(wave_clips, n_clips - w0);
     dw.rows = dw.n * dw.Tp_pad;
     // tensor maps are encoded for d.rows; a smaller last wave only uses a prefix of rows
-    const Acc acc = acc_view(ctx, dw);
-    const float* x = d_audio + (size_t)w0 * stride;
-    int* itc = (int*)ctx->itc.p;
-
-    k_set_int<<<1, 1, 0, st>>>(itc, -1);
-    k_fill<<<(dw.n + 255) / 256, 256, 0, st>>>((float*)ctx->best.p, INFINITY, dw.n);
-    k_pattern_to_float<<<(dw.n * AW_NBITS + 255) / 256, 256, 0, st>>>(
-        d_pattern + (size_t)w0 * AW_NBITS, (float*)ctx->pattern.p, dw.n * AW_NBITS);
-    ctx->launches += 3;
-    AW_LAUNCH_CHECK();
-    if (launch_peak(ctx, x, stride, n_samples, dw.n, (unsigned long long*)ctx->peakx.p, st,
-                    scale_mode == AW_SCALE_SIGNED_MAX ? (int*)ctx->smax.p : nullptr))
-      return 1;
-
-    // ---- pre-STFT, bounds, constant out-of-band waveform (multibit_embedder.py:143-160)
-    nvtxRangePushA("embed:init_stft_bounds_oob");
-    AnaArgs a0 = ana_base(ctx, dw);
-    a0.sig = x; a0.sig_stride = stride; a0.len = n_samples;
-    a0.peak = (unsigned long long*)ctx->peakx.p;
-    a0.mag = (float*)ctx->c0.p; a0.ph = (float2*)ctx->ph_u.p;
-    a0.c = (float*)ctx->c.p; a0.m = (float*)ctx->m.p; a0.v = (float*)ctx->v.p;
-    a0.cbest = (float*)ctx->cbest.p;
-    if (launch_ana<ANA_INIT>(ctx, dw, a0, st)) return 1;
-    SynArgs s0 = syn_base(ctx, dw);
-    s0.amp = (float*)ctx->c0.p; s0.ph = (float2*)ctx->ph_u.p; s0.scale = 1.0f / AW_NFFT;
-    s0.x = x; s0.x_stride = stride; s0.peak_x = (unsigned long long*)ctx->peakx.p;
-    s0.y_oob = (float*)ctx->yoob.p;
-    s0.z_oob = (float*)ctx->zoob.p;
-    if (launch_syn<SYN_OOB>(ctx, dw, s0, st)) return 1;
-    // fp16 loop at 44.1 / 48 kHz: the loop's band-limited transforms run on the tensor cores (spectc.cuh)
-    const bool tc = tc_eligible(ctx, dw);
-    if (tc) {
-      if (tc_prepare_mats(ctx, dw, ctx->h_window.data())) return 1;
-      if (tc_setup_wave(ctx, dw, st)) return 1;
-    }
-    ctx->tc_active = tc;
-    struct TcOff { aw_ctx* c; ~TcOff() { c->tc_active = false; } } tc_off_{ctx};
-    nvtxRangePop();
-
-    // ---- optimisation loop (multibit_embedder.py:95-122)
-    nvtxRangePushA("embed:nadam_loop");
-    auto iteration = [&](bool first) -> int {
-      // fused spectral passes (spec.cuh): y and dpad never leave shared memory
-      if (begin_pass(ctx, dw.n, itc, st)) return 1;
-      if (tc) {
-        if (tc_forward(ctx, dw, acc, st)) return 1;
-      } else {
-        SpecArgs f;
-        memset(&f, 0, sizeof(f));
-        f.amp = (float*)ctx->c.p; f.ph = (float2*)ctx->ph_u.p;
-        f.z_oob = (float*)ctx->zoob.p; f.peak_y = acc.peak_y;
-        f.mag = (float*)ctx->mag.p; f.q = (float2*)ctx->ph_q.p;
-        if (launch_spec<SPEC_FWD>(ctx, dw, f, st)) return 1;
-      }
-      float* lp = d_losses ? d_losses + w0 : nullptr;
-      if (ctx->prec == AW_PREC_BF16) {
-        if (net_forward<__nv_bfloat16>(ctx, dw, acc, sm, st, acc.peak_y)) return 1;
-        if (run_head<__nv_bfloat16>(ctx, dw, (float*)ctx->pattern.p, (float*)ctx->values.p, lp, n_clips, true, st))
-          return 1;
-        if (net_backward<__nv_bfloat16>(ctx, dw, acc, sm, st, true)) return 1;
-      } else if (ctx->prec == AW_PREC_FP16) {
-        if (net_forward<__half>(ctx, dw, acc, sm, st, acc.peak_y)) return 1;
-        if (run_head<__half>(ctx, dw, (float*)ctx->pattern.p, (float*)ctx->values.p, lp, n_clips, true, st))
-          return 1;
-        if (net_backward<__half>(ctx, dw, acc, sm, st, true)) return 1;
-      } else {
-        if (net_forward<float>(ctx, dw, acc, sm, st, acc.peak_y)) return 1;
-        if (run_head<float>(ctx, dw, (float*)ctx->pattern.p, (float*)ctx->values.p, lp, n_clips, true, st))
-          return 1;
-        if (net_backward<float>(ctx, dw, acc, sm, st, true)) return 1;
-      }
-      const double* sp2 = acc.s2_part;
-      int sb2 = p0a_blocks(dw);
-      if (reduce_if_long(ctx, ctx->red_c, sp2, sb2, dw.n, 1, st)) return 1;
-      if (sb2 > 512 && reduce_if_long(ctx, ctx->red_a, sp2, sb2, dw.n, 1, st)) return 1;   // 1 h: 38 760 -> 606 -> 10
-      prof_mark(ctx, st, "clip_scalars");
-      k_clip_scalars<<<(dw.n + 127) / 128, 128, 0, st>>>(acc.peak_y, sp2, sb2, dw.n, (ClipScal*)ctx->scal.p, 0,
-                                                         tc ? (unsigned*)ctx->tc_dmax.p : nullptr, itc);
-      ctx->launches++;
-      AW_LAUNCH_CHECK();
-      if (tc) return tc_backward(ctx, dw, itc, st, (int*)ctx->nonfinite.p + w0, first);
-      SpecArgs b;
-      memset(&b, 0, sizeof(b));
-      b.amp = (float*)ctx->dA.p; b.ph = (float2*)ctx->ph_q.p;
-      b.scal = (ClipScal*)ctx->scal.p; b.u = (float2*)ctx->ph_u.p;
-      b.c = (float*)ctx->c.p; b.m = (float*)ctx->m.p; b.v = (float*)ctx->v.p;
-      b.cbest = (float*)ctx->cbest.p; b.c0 = (float*)ctx->c0.p;
-      b.improved = (int*)ctx->improved.p; b.steps = (NadamStep*)ctx->steps.p; b.it_ptr = itc;
-      b.nonfinite = (int*)ctx->nonfinite.p + w0;
-      b.tol_ratio = (float)pow(10.0, -(double)ctx->tol_db / 20.0);
-      if (launch_spec<SPEC_BWD>(ctx, dw, b, st)) return 1;
-      return 0;
-    };
-    if (use_graph) {
-      // iteration 0 runs eagerly (function attributes, scratch sizes), iteration 1 is captured
-      // without executing, and the graph is replayed for iterations 1 .. iters-1; the iteration
-      // index and all per-clip state live on the device, so every replay is identical work
-      const int64_t l0 = ctx->launches;
-      if (iteration(true)) return 1;
-      const int64_t per_iter = ctx->launches - l0 - (tc ? 1 : 0);
-      AW_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed));
-      const int rc = iteration(false);
-      cudaGraph_t graph = nullptr;
-      const cudaError_t ce = cudaStreamEndCapture(st, &graph);
-      if (rc || ce != cudaSuccess || !graph) {
-        if (graph) cudaGraphDestroy(graph);
-        return rc ? 1 : set_error("aw_embed_batch: stream capture failed: %s", cudaGetErrorString(ce));
-      }
-      cudaGraphExec_t exec = nullptr;
-      if (cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) {
-        cudaGraphDestroy(graph);
-        return set_error("aw_embed_batch: cudaGraphInstantiate failed: %s", cudaGetErrorString(cudaGetLastError()));
-      }
-      for (int it = 1; it < iters; ++it) {
-        if (cudaGraphLaunch(exec, st) != cudaSuccess) {
-          cudaGraphExecDestroy(exec);
-          cudaGraphDestroy(graph);
-          return set_error("aw_embed_batch: cudaGraphLaunch failed: %s", cudaGetErrorString(cudaGetLastError()));
-        }
-      }
-      ctx->launches += per_iter * (iters - 2);      // the captured pass was counted once already
-      cudaGraphExecDestroy(exec);
-      cudaGraphDestroy(graph);
-    } else {
-      for (int it = 0; it < iters; ++it)
-        if (iteration(it == 0)) return 1;
-    }
-    nvtxRangePop();
-    // ---- final synthesis from the best coefficients (multibit_embedder.py:173-192)
-    nvtxRangePushA("embed:final_synthesis");
-    if (begin_pass(ctx, dw.n, nullptr, st)) return 1;
-    SynArgs sf = syn_base(ctx, dw);
-    sf.amp = (float*)ctx->cbest.p; sf.ph = (float2*)ctx->ph_u.p; sf.scale = 1.0f / AW_NFFT;
-    sf.y_oob = (float*)ctx->yoob.p; sf.y = (float*)ctx->y.p; sf.peak_y = acc.peak_y;
-    if (launch_syn<SYN_WAVE>(ctx, dw, sf, st)) return 1;
-    dim3 g(std::min((dw.L + 4095) / 4096, std::max(64, 8192 / dw.n)), dw.n);
-    prof_mark(ctx, st, "final_normalize");
-    k_final_normalize<<<g, 256, 0, st>>>((float*)ctx->y.p, dw.L, acc.peak_y,
-                                         d_scale ? d_scale + w0 : nullptr,
-                                         scale_mode == AW_SCALE_SIGNED_MAX ? (const int*)ctx->smax.p : nullptr,
-                                         d_out + (size_t)w0 * out_stride, out_stride);
-    ctx->launches++;
-    AW_LAUNCH_CHECK();
-    if (d_best_loss)
-      AW_CUDA(cudaMemcpyAsync(d_best_loss + w0, ctx->best.p, (size_t)dw.n * 4,
-                              cudaMemcpyDeviceToDevice, st));
-    ctx->last_n = dw.n; ctx->last_T = dw.T; ctx->last_nb = dw.nb;
-    nvtxRangePop();
+    WaveIO w{};
+    w.x = d_audio + (size_t)w0 * stride; w.stride = stride;
+    w.pattern = d_pattern + (size_t)w0 * AW_NBITS;
+    w.scale = d_scale ? d_scale + w0 : nullptr; w.signed_max = scale_mode == AW_SCALE_SIGNED_MAX;
+    w.out = d_out + (size_t)w0 * out_stride; w.out_stride = out_stride;
+    w.best_loss = d_best_loss ? d_best_loss + w0 : nullptr;
+    w.losses = d_losses ? d_losses + w0 : nullptr; w.n_total = n_clips;
+    w.nonfinite = (int*)ctx->nonfinite.p + w0;
+    if (embed_wave(ctx, dw, dw, w, iters, use_graph, st)) return 1;
   }
   prof_mark(ctx, st, nullptr);
   if (use_graph) {
@@ -1815,7 +1870,8 @@ extern "C" int aw_embed_batch(aw_ctx* ctx, const float* d_audio, int n_clips, in
 // max is reduced over the ranks between the kernel that produces its partials and the kernel that
 // consumes it, and (b) the halo frames of the optimisation variables and of the spectral gradient are
 // refreshed from their owners every iteration.  Results equal the single-GPU run up to the summation
-// order of the float64 statistics.
+// order of the float64 statistics.  The segment runs through detect_pass / embed_wave; the hooks
+// sync_peak, sync_halo and clip_sums are where it differs from a batch of one clip.
 // ---------------------------------------------------------------------------
 static int shard_begin(aw_ctx* ctx, aw_ctx::Shard* sh, const aw_comm* comm, int seg_samples, int seg_first_frame,
                        int own_lo, int own_hi, int total_frames, int sample_rate, Dims* ds, Dims* dn) {
@@ -1835,18 +1891,13 @@ static int shard_begin(aw_ctx* ctx, aw_ctx::Shard* sh, const aw_comm* comm, int 
   AW_REQUIRE(last ? seg_first_frame + ds->T == total_frames : seg_first_frame + ds->T < total_frames + AW_HALO,
              "sharded mode: segment does not fit the clip");
   sh->comm = *comm;
-  sh->T_glob = total_frames;
-  sh->Tp_glob = total_frames / 2;
   sh->e0 = seg_first_frame;
   sh->own_lo = own_lo;
   sh->own_hi = own_hi;
   *dn = *ds;
-  dn->T = own_hi - own_lo;
-  dn->Tp = dn->T / 2;
-  dn->Tp_pad = (dn->Tp + AW_ROW_TILE - 1) / AW_ROW_TILE * AW_ROW_TILE;
-  dn->tiles = dn->Tp_pad / AW_ROW_TILE;
-  dn->rows = dn->Tp_pad;
-  dn->L = AW_HOP * (dn->T - 1);
+  set_frames(dn, own_hi - own_lo);
+  dn->T_clip = total_frames;
+  dn->Tp_clip = total_frames / 2;
   return 0;
 }
 
@@ -1859,31 +1910,11 @@ extern "C" int aw_detect_sharded(aw_ctx* ctx, const float* d_segment, int seg_sa
   aw_ctx::Shard sh;
   Dims ds, dn;
   if (shard_begin(ctx, &sh, comm, seg_samples, seg_first_frame, own_lo, own_hi, total_frames, sample_rate, &ds, &dn)) return 1;
-  if (ensure(ctx->mag, (size_t)ds.T * ds.nb * 4) || ensure_net_ws(ctx, dn, false) ||
-      ensure(ctx->accum, acc_doubles(ds) * 8) || ensure(ctx->peakx, 8))
-    return 1;
-  SparseMel sm;
-  if (get_mel(ctx, ds.bin0, ds.nb, &sm)) return 1;
   ctx->sh = &sh;
   struct Clear { aw_ctx* c; ~Clear() { c->sh = nullptr; } } clear_{ctx};
   nvtxRangePushA("aw_detect_sharded");
   struct Pop { ~Pop() { nvtxRangePop(); } } pop_;
-  const Acc acc = acc_view(ctx, dn);
-  if (begin_pass(ctx, 1, nullptr, st)) return 1;
-  if (launch_peak(ctx, d_segment, seg_samples, seg_samples, 1, (unsigned long long*)ctx->peakx.p, st)) return 1;
-  if (sh_peak_max(ctx, (unsigned long long*)ctx->peakx.p, st)) return 1;        // waveform.py:19 over the whole clip
-  AnaArgs a = ana_base(ctx, ds);
-  a.sig = d_segment; a.sig_stride = seg_samples; a.len = seg_samples;
-  a.peak = (unsigned long long*)ctx->peakx.p;
-  a.mag = (float*)ctx->mag.p;
-  if (launch_ana<ANA_MAG>(ctx, ds, a, st)) return 1;
-  int rc;
-  if (ctx->prec == AW_PREC_BF16)
-    rc = net_forward<__nv_bfloat16>(ctx, dn, acc, sm, st) || run_head<__nv_bfloat16>(ctx, dn, nullptr, d_values, nullptr, 1, false, st);
-  else if (ctx->prec == AW_PREC_FP16)
-    rc = net_forward<__half>(ctx, dn, acc, sm, st) || run_head<__half>(ctx, dn, nullptr, d_values, nullptr, 1, false, st);
-  else
-    rc = net_forward<float>(ctx, dn, acc, sm, st) || run_head<float>(ctx, dn, nullptr, d_values, nullptr, 1, false, st);
+  const int rc = detect_pass(ctx, ds, dn, d_segment, seg_samples, d_values, st);
   prof_mark(ctx, st, nullptr);
   return rc;
 }
@@ -1903,111 +1934,24 @@ extern "C" int aw_embed_sharded(aw_ctx* ctx, const float* d_segment, int seg_sam
   // own output samples: global [256 f0, 256 f1) cut at the clip's length 256 (T - 1)
   const int out_lo = AW_HOP * own_lo, out_hi = std::min(AW_HOP * own_hi, ds.L);
   AW_REQUIRE(out_capacity >= out_hi - out_lo, "aw_embed_sharded: output capacity %lld < %d", (long long)out_capacity, out_hi - out_lo);
-  const size_t sp = (size_t)ds.T * ds.nb;
-  if (ensure(ctx->mag, sp * 4) || ensure_net_ws(ctx, dn, true) || ensure(ctx->accum, acc_doubles(ds) * 8) ||
-      ensure(ctx->ph_u, sp * 8) || ensure(ctx->ph_q, sp * 8) || ensure(ctx->c0, sp * 4) ||
-      ensure(ctx->c, sp * 4) || ensure(ctx->m, sp * 4) || ensure(ctx->v, sp * 4) ||
-      ensure(ctx->cbest, sp * 4) || ensure(ctx->dA, sp * 4) ||
-      ensure(ctx->yoob, (size_t)ds.L * 4) || ensure(ctx->y, (size_t)ds.L * 4) || ensure(ctx->zoob, (size_t)ds.L * 4) ||
-      ensure(ctx->pattern, AW_NBITS * 4) || ensure(ctx->scal, sizeof(ClipScal)) || ensure(ctx->nonfinite, 4) ||
-      ensure(ctx->steps, (size_t)(iters > 0 ? iters : 1) * sizeof(NadamStep)) || ensure(ctx->peakx, 8))
-    return 1;
-  SparseMel sm;
-  if (get_mel(ctx, ds.bin0, ds.nb, &sm)) return 1;
-  std::vector<NadamStep> tab;
-  nadam_table(iters, tab);
-  if (iters > 0)
-    AW_CUDA(cudaMemcpyAsync(ctx->steps.p, tab.data(), tab.size() * sizeof(NadamStep), cudaMemcpyHostToDevice, st));
-  AW_CUDA(cudaMemsetAsync(ctx->nonfinite.p, 0, 4, st));
-  AW_CUDA(cudaMemsetAsync(ctx->dA.p, 0, sp * 4, st));
-  ctx->last_embed_clips = 1;
-  AW_CUDA(cudaStreamSynchronize(st));   // `tab` is pageable host memory
+  if (embed_setup(ctx, ds, dn, 1, iters, st)) return 1;
+  AW_CUDA(cudaMemsetAsync(ctx->dA.p, 0, (size_t)ds.T * ds.nb * 4, st));
   ctx->sh = &sh;
   struct Clear { aw_ctx* c; ~Clear() { c->sh = nullptr; } } clear_{ctx};
   nvtxRangePushA("aw_embed_sharded");
   struct Pop { ~Pop() { nvtxRangePop(); } } pop_;
-
-  const Acc acc = acc_view(ctx, dn);           // peak word at the base; partial-sum arrays of the own frames
-  int* itc = (int*)ctx->itc.p;
-  const int n_base = AW_HOP * seg_first_frame;  // global index of the segment's sample 0
-  k_set_int<<<1, 1, 0, st>>>(itc, -1);
-  k_fill<<<1, 256, 0, st>>>((float*)ctx->best.p, INFINITY, 1);
-  k_pattern_to_float<<<1, 256, 0, st>>>(d_pattern, (float*)ctx->pattern.p, AW_NBITS);
-  ctx->launches += 3;
-  AW_LAUNCH_CHECK();
-  if (launch_peak(ctx, d_segment, seg_samples, seg_samples, 1, (unsigned long long*)ctx->peakx.p, st)) return 1;
-  if (sh_peak_max(ctx, (unsigned long long*)ctx->peakx.p, st)) return 1;
-
-  // ---- pre-STFT, bounds, constant out-of-band waveform of the segment
-  AnaArgs a0 = ana_base(ctx, ds);
-  a0.sig = d_segment; a0.sig_stride = seg_samples; a0.len = seg_samples;
-  a0.peak = (unsigned long long*)ctx->peakx.p;
-  a0.mag = (float*)ctx->c0.p; a0.ph = (float2*)ctx->ph_u.p;
-  a0.c = (float*)ctx->c.p; a0.m = (float*)ctx->m.p; a0.v = (float*)ctx->v.p; a0.cbest = (float*)ctx->cbest.p;
-  if (launch_ana<ANA_INIT>(ctx, ds, a0, st)) return 1;
-  SynArgs s0 = syn_base(ctx, ds);
-  s0.amp = (float*)ctx->c0.p; s0.ph = (float2*)ctx->ph_u.p; s0.scale = 1.0f / AW_NFFT;
-  s0.x = d_segment; s0.x_stride = seg_samples; s0.peak_x = (unsigned long long*)ctx->peakx.p;
-  s0.y_oob = (float*)ctx->yoob.p; s0.z_oob = (float*)ctx->zoob.p;
-  if (launch_syn<SYN_OOB>(ctx, ds, s0, st)) return 1;
-
-  auto net_pass = [&](auto tag) -> int {
-    using AT = decltype(tag);
-    if (net_forward<AT>(ctx, dn, acc, sm, st, acc.peak_y)) return 1;
-    if (run_head<AT>(ctx, dn, (float*)ctx->pattern.p, (float*)ctx->values.p, d_losses, 1, true, st)) return 1;
-    return net_backward<AT>(ctx, dn, acc, sm, st, true);
-  };
-  for (int it = 0; it < iters; ++it) {
-    if (begin_pass(ctx, 1, itc, st)) return 1;
-    SpecArgs f;
-    memset(&f, 0, sizeof(f));
-    f.amp = (float*)ctx->c.p; f.ph = (float2*)ctx->ph_u.p;
-    f.z_oob = (float*)ctx->zoob.p; f.peak_y = acc.peak_y;
-    f.mag = (float*)ctx->mag.p; f.q = (float2*)ctx->ph_q.p;
-    f.pk_lo = out_lo; f.pk_hi = out_hi; f.idx_base = n_base;
-    if (launch_spec<SPEC_FWD>(ctx, ds, f, st)) return 1;
-    if (sh_peak_max(ctx, acc.peak_y, st)) return 1;                      // max |y| over the whole clip
-    int rc;
-    if (ctx->prec == AW_PREC_BF16) rc = net_pass(__nv_bfloat16());
-    else if (ctx->prec == AW_PREC_FP16) rc = net_pass(__half());
-    else rc = net_pass(float());
-    if (rc) return 1;
-    if (sh_reduce_sum(ctx, ctx->red_c, acc.s2_part, p0a_blocks(dn), 1, st)) return 1;   // Euler sum over the clip
-    prof_mark(ctx, st, "clip_scalars");
-    k_clip_scalars<<<1, 128, 0, st>>>(acc.peak_y, sh_red(ctx), 1, 1, (ClipScal*)ctx->scal.p, n_base,
-                                      nullptr, nullptr);
-    ctx->launches++;
-    AW_LAUNCH_CHECK();
-    if (sh_halo_exchange(ctx, (float*)ctx->dA.p, ds.nb, st)) return 1;   // spectral gradient of the halo frames
-    SpecArgs b;
-    memset(&b, 0, sizeof(b));
-    b.amp = (float*)ctx->dA.p; b.ph = (float2*)ctx->ph_q.p;
-    b.scal = (ClipScal*)ctx->scal.p; b.u = (float2*)ctx->ph_u.p;
-    b.c = (float*)ctx->c.p; b.m = (float*)ctx->m.p; b.v = (float*)ctx->v.p;
-    b.cbest = (float*)ctx->cbest.p; b.c0 = (float*)ctx->c0.p;
-    b.improved = (int*)ctx->improved.p; b.steps = (NadamStep*)ctx->steps.p; b.it_ptr = itc;
-    b.nonfinite = (int*)ctx->nonfinite.p;
-    b.tol_ratio = (float)pow(10.0, -(double)ctx->tol_db / 20.0);
-    if (launch_spec<SPEC_BWD>(ctx, ds, b, st)) return 1;
-    if (sh_halo_exchange(ctx, (float*)ctx->c.p, ds.nb, st)) return 1;    // updated coefficients of the halo frames
-  }
-  // ---- final synthesis from the best coefficients, peak over the whole clip, own samples out
-  if (sh_halo_exchange(ctx, (float*)ctx->cbest.p, ds.nb, st)) return 1;
-  if (begin_pass(ctx, 1, nullptr, st)) return 1;
-  SynArgs sf = syn_base(ctx, ds);
-  sf.amp = (float*)ctx->cbest.p; sf.ph = (float2*)ctx->ph_u.p; sf.scale = 1.0f / AW_NFFT;
-  sf.y_oob = (float*)ctx->yoob.p; sf.y = (float*)ctx->y.p; sf.peak_y = acc.peak_y;
-  sf.pk_lo = out_lo; sf.pk_hi = out_hi;
-  if (launch_syn<SYN_WAVE>(ctx, ds, sf, st)) return 1;
-  if (sh_peak_max(ctx, acc.peak_y, st)) return 1;
-  prof_mark(ctx, st, "final_normalize");
-  k_final_normalize<<<dim3(std::min((out_hi - out_lo + 4095) / 4096, 1024), 1), 256, 0, st>>>(
-      (float*)ctx->y.p + out_lo, out_hi - out_lo, acc.peak_y, nullptr, nullptr, d_out_own, out_capacity);
-  ctx->launches++;
-  AW_LAUNCH_CHECK();
-  if (d_best_loss) AW_CUDA(cudaMemcpyAsync(d_best_loss, ctx->best.p, 4, cudaMemcpyDeviceToDevice, st));
+  WaveIO w{};
+  w.x = d_segment; w.stride = seg_samples;
+  w.pattern = d_pattern;
+  w.out = d_out_own; w.out_stride = out_capacity;
+  w.pk_lo = out_lo; w.pk_hi = out_hi;
+  w.idx_base = AW_HOP * seg_first_frame;     // global index of the segment's sample 0
+  w.best_loss = d_best_loss;
+  w.losses = d_losses; w.n_total = 1;
+  w.nonfinite = (int*)ctx->nonfinite.p;
+  // the collectives are host callbacks: no graph replay
+  if (embed_wave(ctx, ds, dn, w, iters, false, st)) return 1;
   if (comm_counts) { comm_counts[0] = sh.n_allreduce; comm_counts[1] = sh.n_allgather; }
-  ctx->last_n = 1; ctx->last_T = ds.T; ctx->last_nb = ds.nb;
   prof_mark(ctx, st, nullptr);
   return 0;
 }
