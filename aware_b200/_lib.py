@@ -81,6 +81,7 @@ SIGNATURES = {
     "aw_attack_cropout": (_i, [_vp, _vp, _i, _i, _i64, _i, _vp, _i64, _vp]),
     "aw_attack_affine": (_i, [_vp, _vp, _i, _i, _i64, _f, _vp, _i64, _f, _vp, _i64, _vp]),
     "aw_attack_spectral_quantize": (_i, [_vp, _vp, _i, _i, _i, _f, _f, _vp, _vp]),
+    "aw_attack_convolve": (_i, [_vp, _vp, _i, _i, _i64, _vp, _i, _i, _vp, _vp, _i64, _vp]),
 }
 
 _lib = None

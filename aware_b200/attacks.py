@@ -10,7 +10,9 @@ coefficients travel.  Upstream's MP3Compression / TimeStretch / PitchShift shell
 ffmpeg / rubberband and have no arithmetic to restate.  MP3 is not provided (`CompressionApprox`
 is an in-repo stand-in); `TimeStretch` / `PitchShift` are defined here as the classical phase
 vocoder (parity unpinned to rubberband), with `desync_attacks()` as the set the evaluation
-driver adds on request.
+driver adds on request.  `Reverb` / `Echo` (room reverberation and echo, a partitioned FFT
+convolution on the GPU) have no upstream counterpart; `room_attacks()` is the set the driver adds
+on request.
 """
 from __future__ import annotations
 
@@ -475,6 +477,150 @@ def desync_attacks():
     and pitch-shift parameters are not recorded in this repository; these values are this project's
     choice: +-10 % tempo and +-2 semitones."""
     return [TimeStretch(0.9), TimeStretch(1.1), PitchShift(-2), PitchShift(2)]
+
+
+# ---- room attacks: reverberation and echo (no upstream counterpart; parity pinned to a float64 convolution)
+CONV_PART = 512                   # partition length of the partitioned convolution
+CONV_MAX_TAPS = 512 * CONV_PART   # 262 144 taps: 512 partitions
+_DECAY_60DB = 6.907755278982137   # ln(1000): amplitude -60 dB
+
+
+def conv_spectra(h) -> np.ndarray:
+    """Partition spectra of impulse responses `h` ([M] or [R, M]) for `Engine.attack_convolve`: complex64
+    [R, K, 513], K = ceil(M / 512), the rfft of each 512-tap partition zero-padded to 1024, computed in float64
+    and rounded to complex64."""
+    h = np.asarray(h, dtype=np.float64)
+    if h.ndim == 1:
+        h = h[None]
+    if h.ndim != 2 or not 1 <= h.shape[1] <= CONV_MAX_TAPS or h.shape[0] < 1:
+        raise ValueError(f"impulse responses must be [M] or [R, M] with 1 <= M <= {CONV_MAX_TAPS} (got {h.shape})")
+    if not np.isfinite(h).all():
+        raise ValueError("impulse responses must be finite")
+    R, M = h.shape
+    K = -(-M // CONV_PART)
+    parts = np.zeros((R, K, CONV_PART), dtype=np.float64)
+    parts.reshape(R, K * CONV_PART)[:, :M] = h
+    return np.fft.rfft(parts, n=2 * CONV_PART, axis=2).astype(np.complex64)
+
+
+def synthetic_rir(rt60: float, sr: int, seed: int) -> np.ndarray:
+    """Exponentially decaying Gaussian noise of length round(rt60 sr) whose amplitude falls by 60 dB over
+    rt60, with h[0] = 1 (direct path), scaled to unit energy; float64 throughout, returned as float32."""
+    M = int(round(rt60 * sr))
+    if not 1 <= M <= CONV_MAX_TAPS:
+        raise ValueError(f"rt60 * sr = {rt60 * sr:g} taps is outside [1, {CONV_MAX_TAPS}]")
+    h = np.random.default_rng(seed).standard_normal(M) * np.exp(-_DECAY_60DB * np.arange(M) / (rt60 * sr))
+    h[0] = 1.0
+    return (h / np.linalg.norm(h)).astype(np.float32)
+
+
+class _Convolve(Attack):
+    """Causal convolution of every clip with an impulse response, truncated to the input's length:
+    y[n] = sum_{m < M} h[m] x[n - m], x[< 0] = 0 (scipy.signal.fftconvolve(x, h)[:N] in float64, float32 out).
+    The GPU runs it as a uniformly partitioned overlap-save convolution (Engine.attack_convolve)."""
+
+    def responses(self, sr: int) -> np.ndarray:
+        """float32 [R, M] impulse responses at sample rate `sr`."""
+        raise NotImplementedError
+
+    def _index(self, n_clips, n_resp, rng):
+        return None
+
+    def apply_batch(self, x, sr, rng=None, engine=None):
+        eng = _eng(engine)
+        key = (int(sr), eng.device.index)
+        if key not in self._spectra:
+            h = self.responses(int(sr))
+            self._spectra[key] = torch.from_numpy(conv_spectra(h)).to(eng.device)
+        spec = self._spectra[key]
+        return eng.attack_convolve(x, spec, self._index(x.shape[0], spec.shape[0], rng))
+
+
+class Reverb(_Convolve):
+    """Room reverberation -- an extension with no upstream counterpart (DESIGN.md section 7).  Each clip is
+    convolved (see `_Convolve`) with one of `n_rirs` synthetic room impulse responses r = 0 .. n_rirs-1:
+    M = round(rt60 sr) taps of np.random.default_rng(seed + r).standard_normal(M) times
+    exp(-6.907755278982137 m / (rt60 sr)) (-60 dB at rt60), then h[0] = 1 (direct path) and h /= ||h||_2,
+    all in float64, cast to float32.  `rir` ([M] or [R, M]) replaces them with the caller's own responses,
+    e.g. a measured one read with `evaluate.read_wav`; rt60 is then not given.  With R > 1 responses every clip draws its own with
+    rng.integers(0, R, n_clips); `index` (one int, or one per clip) fixes the choice instead.  Responses are
+    built per sample rate and cached per (sr, device).  1 <= M <= 262 144."""
+
+    def __init__(self, rt60=None, n_rirs=1, seed=0, rir=None, index=None):
+        if rir is not None:
+            if rt60 is not None:
+                raise ValueError("give either rt60 (synthetic responses) or rir (the caller's own), not both")
+            h = np.asarray(rir, dtype=np.float32)
+            if h.ndim == 1:
+                h = h[None]
+            if h.ndim != 2 or h.shape[0] < 1 or not 1 <= h.shape[1] <= CONV_MAX_TAPS or not np.isfinite(h).all():
+                raise ValueError(f"rir must be finite, [M] or [R, M] with 1 <= M <= {CONV_MAX_TAPS}")
+            self.rir, self.n_rirs, self.rt60 = h, h.shape[0], None
+            self.name = "reverb_rir"
+        else:
+            rt60 = float("nan") if rt60 is None else float(rt60)
+            if not (math.isfinite(rt60) and rt60 > 0):
+                raise ValueError(f"rt60 must be finite and > 0 (got {rt60!r})")
+            if int(n_rirs) < 1:
+                raise ValueError("n_rirs must be >= 1")
+            self.rir, self.n_rirs, self.rt60 = None, int(n_rirs), rt60
+            self.name = f"reverb_{rt60:g}"
+        self.seed = int(seed)
+        if index is not None:
+            index = np.asarray(index)
+            if (index.dtype.kind not in "iu" or index.ndim > 1 or not index.size
+                    or index.min() < 0 or index.max() >= self.n_rirs):
+                raise ValueError(f"index must be integers in [0, {self.n_rirs})")
+        self.index = index
+        self._spectra = {}
+
+    def responses(self, sr: int) -> np.ndarray:
+        if self.rir is not None:
+            return self.rir
+        if not 1 <= round(self.rt60 * sr) <= CONV_MAX_TAPS:
+            raise ValueError(f"rt60 = {self.rt60:g} s at {sr} Hz gives {round(self.rt60 * sr)} taps, outside "
+                             f"[1, {CONV_MAX_TAPS}]")
+        return np.stack([synthetic_rir(self.rt60, sr, self.seed + r) for r in range(self.n_rirs)])
+
+    def _index(self, n_clips, n_resp, rng):
+        if self.index is not None:
+            try:
+                return np.broadcast_to(self.index, (n_clips,)).astype(np.int32)
+            except ValueError:
+                raise ValueError(f"index holds {self.index.size} entries for {n_clips} clips") from None
+        if n_resp == 1:
+            return None
+        rng = rng or np.random.default_rng()
+        return rng.integers(0, n_resp, n_clips).astype(np.int32)
+
+
+class Echo(_Convolve):
+    """A single echo -- an extension with no upstream counterpart (DESIGN.md section 7):
+    y[n] = x[n] + decay x[n - D], D = round(delay sr) >= 1, as the convolution of `_Convolve` with
+    h = [1, 0, ..., 0, decay] (D + 1 taps, not normalised)."""
+
+    def __init__(self, delay=0.05, decay=0.5):
+        self.delay, self.decay = float(delay), float(decay)
+        if not (math.isfinite(self.delay) and self.delay > 0 and math.isfinite(self.decay)):
+            raise ValueError(f"delay must be finite and > 0 and decay finite (got {delay!r}, {decay!r})")
+        self.name = f"echo_{self.delay:g}_{self.decay:g}"
+        self._spectra = {}
+
+    def responses(self, sr: int) -> np.ndarray:
+        """float32 [1, D + 1]: the one impulse response at sample rate `sr`."""
+        D = int(round(self.delay * sr))
+        if not 1 <= D < CONV_MAX_TAPS:
+            raise ValueError(f"delay = {self.delay:g} s at {sr} Hz gives D = {D}, outside [1, {CONV_MAX_TAPS - 1}]")
+        h = np.zeros((1, D + 1), dtype=np.float32)
+        h[0, 0], h[0, D] = 1.0, self.decay
+        return h
+
+
+def room_attacks():
+    """The room attacks `evaluate_clips(..., room=True)` appends.  There is no upstream counterpart, so these
+    parameters are this project's choice: a small and a large room (RT60 0.3 s and 0.7 s, eight synthetic
+    responses each, one drawn per clip) and a 50 ms echo at half amplitude."""
+    return [Reverb(0.3, n_rirs=8, seed=0), Reverb(0.7, n_rirs=8, seed=100), Echo(0.05, 0.5)]
 
 
 def reference_suite():

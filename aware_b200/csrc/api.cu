@@ -16,6 +16,7 @@
 #include "../../include/aware_b200.h"
 #include "attacks.cuh"
 #include "common.cuh"
+#include "conv.cuh"
 #include "fft.cuh"
 #include "gemm.cuh"
 #include "gemm64.cuh"
@@ -126,6 +127,7 @@ struct aw_ctx {
   CUtensorMap tm_act[2][4], tm_dh4[2], tm_ga1024[2], tm_ga512[2], tm_gb1024[2];
   Buf cvt_a, cvt_b;    // aw_gemm bf16 test hook
   Buf stoi_ws;         // aw_stoi_batch workspace
+  Buf conv_x, conv_idx;  // aw_attack_convolve: packed input block spectra, per-clip filter index
   bool stoi_edges_set = false;
   // state of the last embed wave (for aw_embed_state)
   int last_n = 0, last_T = 0, last_nb = 0;
@@ -560,7 +562,8 @@ static std::vector<Buf*> all_bufs(aw_ctx* ctx) {
                  &ctx->values, &ctx->best, &ctx->improved, &ctx->pattern, &ctx->itc, &ctx->steps,
                  &ctx->scal, &ctx->zoob, &ctx->p0coef, &ctx->p0scal, &ctx->hpart, &ctx->hcoef, &ctx->red_a, &ctx->red_b, &ctx->red_c,
                  &ctx->gsc, &ctx->nonfinite, &ctx->smax, &ctx->lowm, &ctx->tc_X, &ctx->tc_dS, &ctx->tc_soob,
-                 &ctx->tc_dX, &ctx->tc_gedge, &ctx->tc_dmax, &ctx->tc_ones, &ctx->stoi_ws};
+                 &ctx->tc_dX, &ctx->tc_gedge, &ctx->tc_dmax, &ctx->tc_ones, &ctx->stoi_ws,
+                 &ctx->conv_x, &ctx->conv_idx};
 }
 
 extern "C" int aw_ctx_destroy(aw_ctx* ctx) {
@@ -2449,6 +2452,50 @@ extern "C" int aw_attack_spectral_quantize(aw_ctx* ctx, const float* d_mag, int 
   prof_mark(ctx, (cudaStream_t)stream, "attack_spec_quant");
   k_spectral_quantize<<<(unsigned)((frames + 3) / 4), 128, 0, (cudaStream_t)stream>>>(d_mag, frames, nbins, k_log,
                                                                                    k_exp, ratio, d_dmag);
+  ctx->launches++;
+  AW_LAUNCH_CHECK();
+  return 0;
+}
+
+// reverberation / echo: causal convolution by partitioned overlap-save (conv.cuh)
+extern "C" int aw_attack_convolve(aw_ctx* ctx, const float* d_in, int n_clips, int n, int64_t in_stride,
+                                  const float* d_spec, int n_filters, int n_parts, const int32_t* filter_of_clip,
+                                  float* d_out, int64_t out_stride, void* stream) {
+  AW_REQUIRE(ctx && d_in && d_spec && d_out, "null argument");
+  AW_REQUIRE(n_clips >= 1 && n_clips <= 65535, "aw_attack_convolve: n_clips must be in [1, 65535] (got %d)", n_clips);
+  // sample indices of the last block reach n + 1535 in 32-bit arithmetic
+  AW_REQUIRE(n >= 1 && n <= INT_MAX - 2048, "aw_attack_convolve: n must be in [1, %d] (got %d)", INT_MAX - 2048, n);
+  AW_REQUIRE(in_stride >= n && out_stride >= n, "aw_attack_convolve: strides must be >= n");
+  AW_REQUIRE(n_filters >= 1, "aw_attack_convolve: n_filters must be >= 1 (got %d)", n_filters);
+  AW_REQUIRE(n_parts >= 1 && n_parts <= AW_CONV_MAXPARTS, "aw_attack_convolve: n_parts must be in [1, %d] (got %d)",
+             AW_CONV_MAXPARTS, n_parts);
+  if (filter_of_clip)
+    for (int i = 0; i < n_clips; ++i)
+      AW_REQUIRE(filter_of_clip[i] >= 0 && filter_of_clip[i] < n_filters,
+                 "aw_attack_convolve: filter_of_clip[%d] = %d must be in [0, %d)", i, filter_of_clip[i], n_filters);
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int nb = (n + AW_CONV_P - 1) / AW_CONV_P;
+  if (ensure(ctx->conv_x, (size_t)n_clips * nb * AW_CONV_SLOTS * sizeof(float2))) return 1;
+  if (filter_of_clip) {
+    if (ensure(ctx->conv_idx, (size_t)n_clips * 4)) return 1;
+    AW_CUDA(cudaMemcpyAsync(ctx->conv_idx.p, filter_of_clip, (size_t)n_clips * 4, cudaMemcpyHostToDevice, st));
+  }
+  ConvArgs a;
+  memset(&a, 0, sizeof(a));
+  a.x = d_in; a.x_stride = in_stride; a.n = n; a.nb = nb;
+  a.X = (float2*)ctx->conv_x.p;
+  a.H = (const float2*)d_spec; a.K = n_parts;
+  a.filter = filter_of_clip ? (const int*)ctx->conv_idx.p : nullptr;
+  a.twiddle = ctx->d_twiddle;
+  a.y = d_out; a.y_stride = out_stride;
+  prof_mark(ctx, st, "conv_fwd");
+  k_conv_fwd<<<dim3((nb + AW_CONV_FWD_BLOCKS - 1) / AW_CONV_FWD_BLOCKS, n_clips), 128, AW_CONV_FWD_SMEM, st>>>(a);
+  ctx->launches++;
+  AW_LAUNCH_CHECK();
+  if (raise_smem_limit(ctx, (const void*)k_conv_mac_inv, AW_CONV_INV_SMEM)) return 1;
+  prof_mark(ctx, st, "conv_mac_inv");
+  k_conv_mac_inv<<<dim3((nb + AW_CONV_R - 1) / AW_CONV_R, n_clips), 512, AW_CONV_INV_SMEM, st>>>(a);
   ctx->launches++;
   AW_LAUNCH_CHECK();
   return 0;

@@ -402,6 +402,27 @@ class Engine:
                                              _ptr(noise), ns, float(sigma), _ptr(out), out.stride(0), _stream()))
         return out
 
+    def attack_convolve(self, x, spec, filter_of_clip=None):
+        """[n, N] -> [n, N]: every clip convolved with its filter, causal and truncated to N samples
+        (scipy.signal.fftconvolve(x, h)[:N]; aw_attack_convolve).  `spec`: complex64 [R, K, 513] on x's device, the
+        partition spectra of `attacks.conv_spectra`; `filter_of_clip`: int [n] in [0, R), or None (filter 0)."""
+        x = self._audio(x)
+        if not (isinstance(spec, torch.Tensor) and spec.device == x.device and spec.dtype == torch.complex64
+                and spec.dim() == 3 and spec.shape[2] == N_BINS_FULL):
+            raise ValueError("expected complex64 partition spectra [n_filters, n_parts, 513] on the device of x")
+        s = torch.view_as_real(spec.contiguous())
+        idx = None
+        if filter_of_clip is not None:
+            idx = np.ascontiguousarray(filter_of_clip, dtype=np.int32)
+            if idx.shape != (x.shape[0],):
+                raise ValueError("filter_of_clip must hold one index per clip")
+        out = self._out_like(x)
+        _lib.check(self.lib.aw_attack_convolve(self._ctx, _ptr(x), x.shape[0], x.shape[1], x.stride(0), _ptr(s),
+                                               s.shape[0], s.shape[1],
+                                               idx.ctypes.data_as(C.c_void_p) if idx is not None else None,
+                                               _ptr(out), out.stride(0), _stream()))
+        return out
+
     def spectral_quantize(self, mag, step_db, floor_db):
         """[n, T, nb] band magnitudes -> (quantised - original) magnitudes (CompressionApprox attack)."""
         n, T, nb = mag.shape

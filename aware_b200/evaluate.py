@@ -12,10 +12,12 @@ on the GPU through the same bit-exact polyphase kernel the `Resample` attack use
 (`parallel.allreduce_counters`).  Upstream's MP3 attack calls ffmpeg and is not run.  Its
 time-stretch and pitch-shift attacks call rubberband; `desync=True` (`--desync`) appends this
 project's phase-vocoder definitions of them (`attacks.desync_attacks()`: time stretch 0.9 / 1.1,
-pitch shift -2 / +2 semitones).  STOI runs on the GPU; PESQ is a third-party package, scored
-when installed and skipped otherwise, like the optional `webrtcvad` gate.
+pitch shift -2 / +2 semitones).  `room=True` (`--room`) appends the reverberation and echo
+attacks (`attacks.room_attacks()`), which have no upstream counterpart.  STOI runs on the GPU;
+PESQ is a third-party package, scored when installed and skipped otherwise, like the optional
+`webrtcvad` gate.
 
-    python -m aware_b200.evaluate <folder with .wav files> [--iters 400] [--seed 0] [--desync]
+    python -m aware_b200.evaluate <folder with .wav files> [--iters 400] [--seed 0] [--desync] [--room]
 """
 from __future__ import annotations
 
@@ -110,20 +112,25 @@ def default_attacks(rng: np.random.Generator):
 
 # ------------------------------------------------------------------------------ the driver
 def evaluate_clips(clips, rates, embedder, detector, attack_list=None, seed: int = 0, keep_audio: bool = False,
-                   desync: bool = False):
+                   desync: bool = False, room: bool = False):
     """clips: list of 1-D float arrays, rates: their sample rates.  Returns a dict with per-attack
     mean BER in percent ('orig' = no attack, as upstream's `rec`), mean SNR, the decoded bits and
     (optionally) the watermarked audio, all for THIS rank's shard when torch.distributed is
     initialised -- the means are over all ranks (counter all-reduce).  `desync` appends
-    `attacks.desync_attacks()` (time stretch / pitch shift) to the attack list."""
+    `attacks.desync_attacks()` (time stretch / pitch shift) to the attack list, `room` appends
+    `attacks.room_attacks()` (reverberation / echo) after them.  The appended attacks draw their random
+    parameters from their own generator, np.random.default_rng((seed, 2)), so they leave the results of
+    the attack list unchanged."""
     from .service import detect_watermark_batch, embed_watermark_batch
     eng = embedder.engine
     A.set_engine(eng)
     rng = np.random.default_rng(seed)
-    attack_list = default_attacks(rng) if attack_list is None else attack_list
-    if desync:
-        attack_list = list(attack_list) + A.desync_attacks()
-    names = ["orig"] + [a.name for a in attack_list]
+    attack_list = default_attacks(rng) if attack_list is None else list(attack_list)
+    # the optional attacks draw from a generator of their own (Reverb picks a response per clip), so the
+    # draws of the attack list, and with them its results, are the same with or without them
+    extra = (A.desync_attacks() if desync else []) + (A.room_attacks() if room else [])
+    extra_rng = np.random.default_rng((seed, 2))
+    names = ["orig"] + [a.name for a in attack_list + extra]
     world = torch.distributed.get_world_size() if torch.distributed.is_initialized() else 1
     rank = torch.distributed.get_rank() if torch.distributed.is_initialized() else 0
     bits_all = np.random.default_rng(seed + 1).integers(0, 2, size=(len(clips), 20), dtype=np.int32)
@@ -186,6 +193,11 @@ def evaluate_clips(clips, rates, embedder, detector, attack_list=None, seed: int
         A.run_suite(attack_list, y, TARGET_SR,
                     lambda a_i, z: detect_watermark_batch(z, TARGET_SR, detector, bits, counters[a_i + 1]),
                     rng=rng, engine=eng)
+        if extra:
+            first = 1 + len(attack_list)
+            A.run_suite(extra, y, TARGET_SR,
+                        lambda a_i, z: detect_watermark_batch(z, TARGET_SR, detector, bits, counters[first + a_i]),
+                        rng=extra_rng, engine=eng)
     allreduce_counters(counters, sums)
     c = counters.cpu().numpy()
     ber = {nm: (100.0 * c[k, 0] / c[k, 1] if c[k, 1] else float("nan")) for k, nm in enumerate(names)}
@@ -204,6 +216,8 @@ def main(argv=None):
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--desync", action="store_true",
                     help="also run the time-stretch (0.9, 1.1) and pitch-shift (-2, +2 semitones) attacks")
+    ap.add_argument("--room", action="store_true",
+                    help="also run the reverberation (RT60 0.3 s, 0.7 s) and echo (50 ms, 0.5) attacks")
     args = ap.parse_args(argv)
     from .utils.models import load
     paths = sorted(os.path.join(args.folder, f) for f in os.listdir(args.folder) if f.lower().endswith(".wav"))
@@ -214,7 +228,8 @@ def main(argv=None):
     embedder, detector = load()
     embedder.num_iterations = args.iters
     embedder.verbose = False
-    res = evaluate_clips(list(clips), list(rates), embedder, detector, seed=args.seed, desync=args.desync)
+    res = evaluate_clips(list(clips), list(rates), embedder, detector, seed=args.seed, desync=args.desync,
+                         room=args.room)
     for name, v in res["ber_percent"].items():
         logger.info(f"{name}: mean: {v:.4f}")
     logger.info(f"snr: mean: {res['snr_db_mean']:.2f} dB over {res['n_clips']} clips")

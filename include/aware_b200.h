@@ -257,6 +257,19 @@ int aw_attack_affine(aw_ctx* ctx, const float* d_in, int n_clips, int n, int64_t
 int aw_attack_spectral_quantize(aw_ctx* ctx, const float* d_mag, int n_clips, int n_frames, int nbins,
                                 float step_db, float floor_db, float* d_dmag, void* stream);
 
+/* ---- reverberation / echo attacks (no upstream counterpart; DESIGN.md section 7).
+ * out = causal convolution of every clip with its filter, truncated to n samples (DESIGN section 7):
+ * y[t] = sum_{m < M} h[m] x[t - m], x[< 0] = 0, by uniformly partitioned overlap-save (512-sample
+ * partitions, 1024-point transforms).
+ * d_spec: complex64 [n_filters][n_parts][513], the rfft of each 512-tap partition zero-padded to 1024
+ * (host-computed in float64, rounded to complex64); 1 <= n_parts <= 512.
+ * filter_of_clip: HOST int32 [n_clips] in [0, n_filters), or NULL (every clip uses filter 0);
+ * validated here and uploaded with cudaMemcpyAsync.  1 <= n <= INT_MAX - 2048, strides >= n, n_clips <= 65535.
+ * Does not synchronise the stream; a clip's result does not depend on the rest of the batch. */
+int aw_attack_convolve(aw_ctx* ctx, const float* d_in, int n_clips, int n, int64_t in_stride,
+                       const float* d_spec, int n_filters, int n_parts, const int32_t* filter_of_clip,
+                       float* d_out, int64_t out_stride, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
